@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- gates/sec and effective HBM GB/s of the state-vector apply path (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--qubits n] [--precision 32|64]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--qubits n] [--precision 32|64] [--dump-outputs DIR]
 
 A "step" is one execution of the whole fused circuit (all passes) on the device-resident state.
 Workload at every N: random_layered(34 q, depth 20, seed 12345), f32 -- BASELINE.json's "34q (1/2/4/8 B200)"
@@ -29,6 +29,8 @@ sys.path.insert(0, ROOT)
 
 SEED = 12345
 DEPTH = 20
+# --dump-outputs: 256 runs of 2^13 consecutive amplitudes = 2^21 amplitudes, 16 MiB (f32) or 32 MiB (f64), plus 16 MiB of indices
+DUMP_RUNS, DUMP_RUN_BITS = 256, 13
 
 
 def load_peaks():
@@ -218,6 +220,23 @@ def run_reference_arm(args):
 
 
 # ------------------------------------------------------------------------------------------------- our arm
+def dump_outputs(out_dir, sim):
+    """The state the last timed step left, as a fixed sample: DUMP_RUNS runs of 2^DUMP_RUN_BITS consecutive logical
+    amplitudes at seeded positions (the whole state when it is no larger).  state.npy holds one (re, im) row per
+    amplitude in the device precision, state_index.npy the logical index of each row."""
+    import numpy as np
+    n = sim.num_qubits
+    bits = min(DUMP_RUN_BITS, n)
+    runs = 1 << (n - bits)
+    picked = np.arange(runs) if runs <= DUMP_RUNS else np.sort(np.random.default_rng(SEED).choice(runs, DUMP_RUNS, replace=False))
+    firsts = [int(r) << bits for r in picked]
+    amps = np.concatenate([sim.state_native(f, 1 << bits) for f in firsts]).reshape(-1, 2)
+    index = np.concatenate([np.arange(f, f + (1 << bits), dtype=np.float64) for f in firsts])
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "state.npy"), amps)
+    np.save(os.path.join(out_dir, "state_index.npy"), index)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -230,6 +249,8 @@ def run_ours(args):
     if world != args.gpus:
         if world == 1 and args.gpus > 1:
             raise SystemExit("launch multi-GPU runs with torch.distributed.run (one rank per GPU)")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs reads the state of a single-GPU run")
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: the product has no CPU path")
     torch.cuda.set_device(local_rank)
@@ -363,6 +384,8 @@ def run_ours(args):
     circ, sim, plan, pst = m["circ"], m["sim"], m["plan"], m["pst"]
     ms_per_step, value, wall_ms, xch_ms, clocks, roofline = (m[k] for k in ("ms_per_step", "value", "wall_ms", "xch_ms", "clocks", "roofline"))
     n_loc_amps = m["n_loc_amps"]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, sim)
 
     # ---- e2e: QASM text (host) -> parse -> plan (H2D) -> |0> -> execute -> result to host memory
     e2e = None
@@ -516,7 +539,13 @@ def main():
     ap.add_argument("--fused", type=int, default=0, help="multi-GPU A/B: exchange flavour, 0 = default (fused peer scatter; pipelined at 2 GPUs), 1 = fused peer scatter (direct: victims anywhere), 2 = NCCL all-to-all, 3 = pipelined copy-engine exchange, 4 = round-1 fused flavour")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--res4", type=int, default=0, help="planner A/B: qsb_options_t.reserved[4] (1 = vector-bit phases not deferred, 2 = no 2x2 products, 3 = no Hadamard-like slot form, 4 = no merged phase runs, 5 = h cx h stays as it is, 6 = CX -> controlled phase with an h on one side too)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a seeded sample of the state the last one "
+                                                          "computed to DIR/state.npy and its logical indices to DIR/state_index.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

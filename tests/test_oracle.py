@@ -1,8 +1,7 @@
-"""Pin the CPU checker: restatement (oracle/qsim_oracle.c) vs the unmodified reference build
-(oracle/_ref) and vs the committed golden vectors.  CPU only."""
+"""Pin the CPU checker: restatement (oracle/qsim_oracle.c) vs the outputs of the unmodified reference
+program stored in tests/golden/ (oracle/make_golden.py) and vs circuits it runs itself.  CPU only."""
 import math
 import os
-import tempfile
 
 import numpy as np
 import pytest
@@ -10,8 +9,21 @@ import pytest
 import helpers
 from gpu_quantum_simulator_b200 import circuits
 
-needs_ref = pytest.mark.skipif(not helpers.have_ref(), reason="oracle/_ref not built")
-needs_refdir = pytest.mark.skipif(not os.path.isdir(helpers.REFERENCE_DIR), reason="/root/reference absent")
+
+def golden(name):
+    return helpers.load_case(os.path.join(helpers.GOLDEN, name + ".npz"))
+
+
+def golden_with_note(note):
+    return [os.path.basename(p)[:-4] for p in helpers.golden_cases() if helpers.load_case(p)[3] == note]
+
+
+def oracle_run_text(text, tmp_path, phi=0.0):
+    """The restatement on a QASM file with this text, times the global phase e^{i phi}."""
+    path = tmp_path / "c.qasm"
+    path.write_bytes(text.encode())
+    n, v = helpers.oracle_run_file(path)
+    return n, v * complex(math.cos(phi), math.sin(phi))
 
 
 def test_known_answers_bell():
@@ -20,50 +32,41 @@ def test_known_answers_bell():
     assert v[0] == r and v[3] == r and v[1] == 0 and v[2] == 0
 
 
-@needs_refdir
-@needs_ref
 @pytest.mark.parametrize("name", ["entanglement.qasm", "grover_3_18.qasm"])
-def test_restatement_equals_reference_on_shipped_files(name):
-    path = os.path.join(helpers.REFERENCE_DIR, name)
-    n1, a = helpers.oracle_run_file(path)
-    n2, b = helpers.ref_run_file(path)
-    assert n1 == n2
-    assert np.array_equal(a, b), "restatement must be bit-identical to quantum_simulator.c"
+def test_restatement_equals_reference_on_shipped_files(name, tmp_path):
+    """The reference's two circuit files, rewritten from the stored fixture with CRLF line ends as shipped, through
+    the restatement's file reader: bit-identical to the reference's own run of them."""
+    circ, n, amps, _ = golden(name[:-5])
+    n1, a = oracle_run_text(circuits.to_qasm(circ, n).replace("\n", "\r\n"), tmp_path)
+    assert n1 == n
+    assert np.array_equal(a, amps), "restatement must be bit-identical to quantum_simulator.c"
 
 
-@needs_refdir
-@needs_ref
 def test_grover_known_values():
-    _, v = helpers.ref_run_file(os.path.join(helpers.REFERENCE_DIR, "grover_3_18.qasm"))
+    _, _, v, _ = golden("grover_3_18")
     p = np.abs(v) ** 2
     assert abs(p[3] - 0.49959115777166263) < 1e-15 and abs(p[18] - 0.49959115777166119) < 1e-15
     assert set(np.argsort(p)[-2:]) == {3, 18}
 
 
-@needs_ref
-@pytest.mark.parametrize("n,ng,seed", [(1, 20, 0), (2, 50, 1), (6, 300, 2), (11, 500, 3), (16, 120, 4)])
-def test_restatement_equals_reference_on_random_reference_gate_circuits(n, ng, seed):
-    circ = circuits.random_reference_gates(n, ng, seed)
-    with tempfile.NamedTemporaryFile("w", suffix=".qasm", delete=False) as f:
-        f.write(circuits.to_qasm(circ, n))
-        path = f.name
-    try:
-        _, a = helpers.oracle_run_file(path)
-        _, b = helpers.ref_run_file(path)
-    finally:
-        os.unlink(path)
-    assert np.array_equal(a, b)
+@pytest.mark.parametrize("name", golden_with_note("reference gate set"))
+def test_restatement_equals_reference_on_random_reference_gate_circuits(name, tmp_path):
+    circ, n, amps, _ = golden(name)
+    _, a = oracle_run_text(circuits.to_qasm(circ, n), tmp_path)
+    assert np.array_equal(a, amps)
     assert np.array_equal(a, helpers.oracle_run_circuit(circ, n))
 
 
-@needs_ref
 @pytest.mark.parametrize("n,ng,seed", [(3, 60, 5), (8, 250, 6), (12, 300, 7)])
-def test_superset_gates_match_reference_through_identities(n, ng, seed):
+def test_superset_gates_match_reference_through_identities(n, ng, seed, tmp_path):
     """rx/ry/y/cz/cp/swap/ccx are not in the reference's gate set: the restatement's native
-    versions must equal the reference run on the exact respelling (times the dropped phase)."""
+    versions must equal the reference run on the exact respelling (times the dropped phase).  The
+    restatement stands in for the reference on the respelling, a file in the reference's gate set:
+    the test above pins it bit-identical to the reference's stored outputs on such files."""
     circ = circuits.random_superset(n, ng, seed)
     a = helpers.oracle_run_circuit(circ, n)
-    b = helpers.ref_run_circuit(circ, n)
+    text, phi = circuits.to_reference_qasm(circ, n)
+    _, b = oracle_run_text(text, tmp_path, phi)
     assert np.max(np.abs(a - b)) < 1e-13
 
 
