@@ -6,8 +6,10 @@ compute happens in the hand-written CUDA library; there is no CPU or PyTorch
 fallback -- importing works anywhere, running needs a CUDA device.
 """
 from ._lib import lib, QsbError, Gate, Options, RunStats, F32, F64, MODE_TILED, MODE_SWEEP, MODE_DENSE  # noqa: F401
-from .simulator import Simulator, parse_qasm_file, parse_qasm_string, gates_from_circuit, plan_dry_run, sample_uniform  # noqa: F401
+from .simulator import (Simulator, parse_qasm_file, parse_qasm_string, gates_from_circuit, plan_dry_run, sample_uniform,  # noqa: F401
+                        expectation_dry_run, pauli_masks)
 from . import circuits  # noqa: F401
 
 __all__ = ["Simulator", "parse_qasm_file", "parse_qasm_string", "gates_from_circuit", "plan_dry_run", "sample_uniform",
+           "expectation_dry_run", "pauli_masks",
            "circuits", "lib", "QsbError", "Gate", "Options", "RunStats", "F32", "F64", "MODE_TILED", "MODE_SWEEP", "MODE_DENSE"]

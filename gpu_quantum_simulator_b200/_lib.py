@@ -62,6 +62,10 @@ SYMBOLS = {
     "qsb_cdf": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64]),
     "qsb_sample": (C.c_int, [C.c_void_p, C.c_uint64, C.c_int, C.c_void_p]),
     "qsb_sample_uniform": (C.c_double, [C.c_uint64, C.c_int]),
+    "qsb_expectation_pauli": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "qsb_pauli_from_string": (C.c_int, [C.c_char_p, C.c_int, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+    "qsb_expectation_dry_run": (C.c_int, [C.c_int, C.POINTER(Options), C.c_void_p, C.c_void_p, C.c_size_t,
+                                          C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     "qsb_save_state": (C.c_int, [C.c_void_p, C.c_char_p]),
     "qsb_load_state": (C.c_int, [C.c_void_p, C.c_char_p]),
     "qsb_comm_unique_id": (C.c_int, [C.c_void_p]),

@@ -10,6 +10,8 @@
  *   <number_of_measurement> > 0 with --shots: "MEASUREMENT: <bits> (%ld)" (quantum_simulator.c:68-73)
  *   --save-state FILE / --load-state FILE   raw shard + qubit map after / before the circuit (checkpoint;
  *                       the reference keeps the state only in memory, quantum_simulator.c:75)
+ *   --expect "Z0 Z1"    (repeatable) <psi|P|psi> of a Pauli string after the circuit, computed on the device:
+ *                       one "EXPECTATION <text>: %.17g" line per flag, in flag order, after the --profile line
  *   --plan-only [--gpus N]   host-side fusion only (no GPU needed): one JSON line with the passes, rounds, ops and
  *                       qubit exchanges the circuit would run as on N ranks, instead of running it
  * Errors go to stdout followed by exit(1), like the reference (:56,:129,:213-219).
@@ -57,6 +59,7 @@ int main(int argc, char **argv)
     long num_m = 0;
     int precision = 32, dump = 0, shots = 0, prec_out = 0, profile = 0, sweep = 0, have_m = 0, plan_only = 0, gpus = 1;
     unsigned long long seed = 0; int have_seed = 0;
+    const char **expect = (const char **)calloc((size_t)argc, sizeof(char *)); int n_expect = 0;
     for (int i = 1; i < argc; i++) {
         if (!strcmp(argv[i], "--precision") && i + 1 < argc) precision = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--dump-amplitudes")) dump = 1;
@@ -70,6 +73,7 @@ int main(int argc, char **argv)
         else if (!strcmp(argv[i], "--plan-only")) plan_only = 1;
         else if (!strcmp(argv[i], "--gpus") && i + 1 < argc) gpus = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--sweep")) sweep = 1;
+        else if (!strcmp(argv[i], "--expect") && i + 1 < argc) expect[n_expect++] = argv[++i];
         else if (!file) file = argv[i];
         else if (!have_m) { num_m = atol(argv[i]); have_m = 1; }
     }
@@ -117,6 +121,16 @@ int main(int argc, char **argv)
                (unsigned long long)st.bytes_moved, st.device_ms > 0 ? st.bytes_moved / st.device_ms * 1e-6 : 0.0,
                st.device_ms > 0 ? st.source_gates / st.device_ms * 1e3 : 0.0);
     }
+    if (n_expect) {   /* one call for all terms: they share the sweeps over the state */
+        uint64_t *ex = (uint64_t *)malloc(sizeof(uint64_t) * 2 * n_expect);
+        double *ev = (double *)malloc(sizeof(double) * n_expect);
+        if (!ex || !ev) { printf("Malloc error\n"); return 1; }
+        for (int k = 0; k < n_expect && !rc; k++) rc = qsb_pauli_from_string(expect[k], nq, &ex[k], &ex[n_expect + k]);
+        if (!rc) rc = qsb_expectation_pauli(s, ex, ex + n_expect, (size_t)n_expect, ev);
+        if (rc) { printf("%s\n", qsb_last_error()); return 1; }
+        for (int k = 0; k < n_expect; k++) printf("EXPECTATION %s: %.17g\n", expect[k], ev[k]);
+        free(ex); free(ev);
+    }
     const unsigned long long N = 1ULL << nq;
     if (dump || dump_bin) {
         const unsigned long long chunk = 1ULL << 20;
@@ -154,5 +168,6 @@ int main(int argc, char **argv)
     }
     qsb_destroy(s);
     qsb_free(gates);
+    free(expect);
     return 0;
 }

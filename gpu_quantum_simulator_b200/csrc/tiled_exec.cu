@@ -180,6 +180,17 @@ int tiled_comm_allreduce_sum_u64(qsb_sim *s, void *dbuf, size_t count)
     return QSB_OK;
 }
 
+/* one send / receive pair with `peer` (expectation values: the partner shard of terms that flip rank bits) */
+int tiled_comm_sendrecv(qsb_sim *s, const void *dsend, void *drecv, size_t bytes, int peer)
+{
+    if (!s->comm) { qsb_set_error("sharded readout needs qsb_comm_init first"); return QSB_ERR_COMM; }
+    QSB_NCCL(g_nccl.GroupStart());
+    QSB_NCCL(g_nccl.Send(dsend, bytes, 1 /* ncclUint8 */, peer, (qsb_nccl_comm_t)s->comm, s->stream));
+    QSB_NCCL(g_nccl.Recv(drecv, bytes, 1, peer, (qsb_nccl_comm_t)s->comm, s->stream));
+    QSB_NCCL(g_nccl.GroupEnd());
+    return QSB_OK;
+}
+
 void tiled_comm_destroy(qsb_sim *s)
 {
     if (s->peers_ok) {

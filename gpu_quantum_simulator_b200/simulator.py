@@ -97,6 +97,29 @@ def plan_dry_run(num_qubits, gates, precision=F32, low_bits=0, world_size=1, ran
     return st.as_dict()
 
 
+def pauli_masks(paulis, num_qubits):
+    """A Pauli string ("X0 Z3 Y5"; "" or "I" = identity) or a list of them -> (x, z) uint64 arrays of logical
+    masks.  The format is defined once, in qsb_pauli_from_string."""
+    texts = [paulis] if isinstance(paulis, str) else list(paulis)
+    x = np.zeros(len(texts), dtype=np.uint64)
+    z = np.zeros(len(texts), dtype=np.uint64)
+    xm, zm = C.c_uint64(), C.c_uint64()
+    for k, t in enumerate(texts):
+        check(lib.qsb_pauli_from_string(t.encode(), num_qubits, C.byref(xm), C.byref(zm)))
+        x[k], z[k] = xm.value, zm.value
+    return x, z
+
+
+def expectation_dry_run(num_qubits, paulis, precision=F32, world_size=1):
+    """Host-only: {"sweeps", "exchanges"} that Simulator.expectation would run for these Pauli strings from the
+    identity qubit layout (sweeps = reads of the local shard, exchanges = partner shards fetched)."""
+    x, z = pauli_masks(paulis, num_qubits)
+    o = _options(precision, MODE_TILED, 0, 0, world_size, -1)
+    sw, ex = C.c_uint32(), C.c_uint32()
+    check(lib.qsb_expectation_dry_run(num_qubits, C.byref(o), x.ctypes.data, z.ctypes.data, x.size, C.byref(sw), C.byref(ex)))
+    return {"sweeps": sw.value, "exchanges": ex.value}
+
+
 class Plan:
     def __init__(self, sim, handle):
         self.sim, self.handle = sim, handle
@@ -257,6 +280,15 @@ class Simulator:
         out = np.empty(shots, dtype=np.uint64)
         check(lib.qsb_sample(self._h, seed, shots, out.ctypes.data))
         return out
+
+    def expectation(self, paulis):
+        """<psi|P|psi> of a Pauli string ("Z0 Z1", "X0 Y2", "" = identity) as a float, or of a list of them as a
+        float64 array, computed on the device without copying the state out.  On a sharded state every rank calls
+        it with the same strings and receives every value."""
+        x, z = pauli_masks(paulis, self.num_qubits)
+        out = np.empty(x.size, dtype=np.float64)
+        check(lib.qsb_expectation_pauli(self._h, x.ctypes.data, z.ctypes.data, x.size, out.ctypes.data))
+        return float(out[0]) if isinstance(paulis, str) else out
 
     def save_state(self, path):
         """Dump this rank's shard (device dtype, physical order) with its qubit map; one file per rank."""

@@ -182,6 +182,30 @@ int qsb_sample(qsb_t *s, uint64_t seed, int shots, uint64_t *out);
  * measurement()'s search on a CDF of its own. */
 double qsb_sample_uniform(uint64_t seed, int k);
 
+/* ---- observables ------------------------------------------------------------
+ * A Pauli string is a pair of masks over LOGICAL qubits: x bit q = X on qubit q, z bit q = Z on qubit q, both
+ * = Y (Y = i X Z = [[0, -i], [i, 0]]).  Its action on an amplitude vector, which tests and callers share:
+ *     (P a)_j = i^{popc(x & z)} * (-1)^{popc((j ^ x) & z)} * a_{j ^ x}
+ * and the value returned is <psi|P|psi> = sum_j conj(a_j) (P a)_j, real, in fp64, on the state as stored (no
+ * renormalisation: x = z = 0 gives the norm).
+ *
+ * Evaluated on the device in tile sweeps: terms whose X parts differ only inside one tile of the state share a
+ * single read of it (diagonal terms all share one sweep; n single-qubit X terms take about n / 8), partial sums
+ * are reduced in a fixed order (repeated calls return identical bits).  Cost: one read of the local shard per
+ * sweep; on a sharded state, one copy of a partner shard per distinct pattern of X on rank qubits. */
+/* out[k] = <psi| P_k |psi> for Pauli strings given as logical masks (x: X or Y, z: Z or Y).
+ * Blocking.  Does not change the state or the qubit layout.  On a sharded state every rank
+ * calls it with the same terms (collective), and every rank receives every value. */
+int qsb_expectation_pauli(qsb_t *s, const uint64_t *x, const uint64_t *z, size_t nterms, double *out);
+/* "X0 Z3 Y5" -> masks.  Tokens are [IXYZ]<qubit>, separated by whitespace.
+ * "" or "I" is the identity.  A repeated qubit or an unknown letter gives QSB_ERR_PARSE.
+ * A qubit >= num_qubits gives QSB_ERR_ARG. */
+int qsb_pauli_from_string(const char *text, int num_qubits, uint64_t *x, uint64_t *z);
+/* Host only, no device: the number of state sweeps and shard exchanges that qsb_expectation_pauli
+ * would run for these terms from the identity layout.  The counterpart of qsb_plan_dry_run. */
+int qsb_expectation_dry_run(int num_qubits, const qsb_options_t *opt, const uint64_t *x, const uint64_t *z,
+                            size_t nterms, uint32_t *sweeps, uint32_t *exchanges);
+
 /* ---- shard dump / reload ----------------------------------------------------
  * The reference keeps the state only in memory (quantum_simulator.c:75 frees it
  * at exit); long sharded runs want a checkpoint.  File = 128-byte header (magic
