@@ -51,6 +51,8 @@ int tiled_comm_sendrecv(qsb_sim *s, const void *dsend, void *drecv, size_t bytes
 #define EXP_UB 4                    /* log2(EXP_NU) */
 #define EXP_T_F32 (1 + EXP_TB + EXP_UB)   /* 12: pack lane + thread + unit bits */
 #define EXP_T_F64 (EXP_TB + EXP_UB)       /* 11 */
+/* a sweep reads pb[0..T-1], which exist because every shard has nloc >= tiled_min_local_bits() = QSB_T_* local bits */
+static_assert(EXP_T_F32 <= QSB_T_F32 && EXP_T_F64 <= QSB_T_F64, "the expectation tile must fit the smallest shard");
 #define EXP_TILE_UNITS (EXP_THREADS * EXP_NU)
 #define EXP_KMAX 512                /* terms per launch: 32 KiB tile + 4 x 512 fp64 accumulators = 48 KiB */
 #define EXP_CTAS_PER_SM(f32) ((f32) ? 4 : 3)   /* f64: the tile in registers and fp64 addresses need more than 128 registers */
@@ -200,7 +202,7 @@ __global__ void k_expect_finish(const double *partial, int nblk, int K, const Ex
     double acc = 0.0;
     for (int b = 0; b < nblk; b++) acc += partial[(size_t)b * K + j];
     acc *= weight;
-    res[terms[j].out] = (terms[j].flags & EXP_NEG) ? -acc : acc;
+    res[terms[j].out] = (terms[j].flags & EXP_NEG) ? 0.0 - acc : acc;   /* not -acc: a zero value stays +0.0 */
 }
 
 /* ================================================================================================ host */

@@ -217,11 +217,11 @@ __global__ void __launch_bounds__(RB) k_chunk_scan(double *p, uint64_t count, co
 }
 
 template <typename R>
-__global__ void k_probs_order(const R *st, double *out, uint64_t first, uint64_t count, OrderArg P, uint64_t loc_mask)
+__global__ void k_probs_order(const R *st, double *out, uint64_t first, uint64_t count, OrderArg P)
 {
     uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= count) return;
-    out[k] = prob_at(st, order_to_phys(first + k, P, 0, P.n) & loc_mask);
+    out[k] = prob_at(st, order_to_phys(first + k, P, 0, P.n));
 }
 
 /* ================================================================================================ host */
@@ -236,46 +236,42 @@ static OrderArg order_arg(const qsb_sim *s, int *bits)
     return P;
 }
 
-static bool sim_range_is_local(const qsb_sim *s, uint64_t first, uint64_t count)
-{
-    if (s->g == 0 || count == 0) return true;
-    uint64_t lmask = 0, want = 0;
-    for (int q = 0; q < s->n; q++) if (s->perm.pos[q] >= s->nloc) {
-        lmask |= 1ULL << q;
-        if ((s->rank >> (s->perm.pos[q] - s->nloc)) & 1) want |= 1ULL << q;
-    }
-    const int lowest = __builtin_ctzll(lmask);
-    for (uint64_t i = first; i < first + count; i = ((i >> lowest) + 1) << lowest) if ((i & lmask) != want) return false;
-    return ((first + count - 1) & lmask) == want;
-}
-
+/* Chunks sit at fixed multiples of `chunk` in the logical index space, so every value is produced by the same
+ * additions whatever (first, count) asks for: cdf(first, count) is cdf(0, 2^n)[first, first + count) bit for bit.
+ * Chunks wholly below `first` only advance the carry (|a|^2, block totals, offsets; no scan, no copy). */
 extern "C" int qsb_cdf(qsb_t *s, double *cdf, uint64_t first, uint64_t count)
 {
     if (!s || (!cdf && count)) { qsb_set_error("qsb_cdf: null argument"); return QSB_ERR_ARG; }
     const uint64_t total = 1ULL << s->n;
     if (first > total || count > total - first) { qsb_set_error("range [%llu, +%llu) exceeds 2^%d amplitudes", (unsigned long long)first, (unsigned long long)count, s->n); return QSB_ERR_ARG; }
-    if (!sim_range_is_local(s, first, count)) { qsb_set_error("range is not owned by rank %d", s->rank); return QSB_ERR_ARG; }
+    if (s->g) {
+        qsb_set_error("qsb_cdf: the state is sharded over %d ranks and the prefix sum below this rank's indices lives on the others; "
+                      "draw shots with qsb_sample, which works on sharded states", s->world);
+        return QSB_ERR_ARG;
+    }
+    if (count == 0) return QSB_OK;
     QSB_CUDA(cudaSetDevice(s->device));
-    /* order = logical index; the rank bits of the address (sharded state) are masked off */
-    OrderArg P; memset(&P, 0, sizeof P);
-    P.n = s->n;
-    for (int q = 0; q < s->n; q++) P.pos[q] = s->perm.pos[q];
-    const uint64_t loc_mask = (1ULL << s->nloc) - 1;
+    int bits = 0;
+    const OrderArg P = order_arg(s, &bits);   /* one GPU: order = logical index */
     const uint64_t chunk = std::min<uint64_t>(s->staging_bytes / 8, (uint64_t)CB * 1024);   /* <= 1024 CTA totals per chunk */
     double *d_p = (double *)s->staging;
     double *d_blk = (double *)((char *)s->d_scratch + 131072);        /* 1024 doubles */
     double *d_carry = (double *)((char *)s->d_scratch + 131072 + 8192);
     QSB_CUDA(cudaMemsetAsync(d_carry, 0, sizeof(double), s->stream));
-    for (uint64_t off = 0; off < count; off += chunk) {
-        const uint64_t c = std::min(chunk, count - off);
+    const uint64_t end = first + count;
+    for (uint64_t c0 = 0; c0 < end; c0 += chunk) {
+        const uint64_t c = std::min(chunk, end - c0);
         const unsigned nblk = (unsigned)((c + CB - 1) / CB);
-        if (s->prec == QSB_F32) k_probs_order<float><<<(unsigned)((c + 255) / 256), 256, 0, s->stream>>>((const float *)s->state, d_p, first + off, c, P, loc_mask);
-        else k_probs_order<double><<<(unsigned)((c + 255) / 256), 256, 0, s->stream>>>((const double *)s->state, d_p, first + off, c, P, loc_mask);
+        if (s->prec == QSB_F32) k_probs_order<float><<<(unsigned)((c + 255) / 256), 256, 0, s->stream>>>((const float *)s->state, d_p, c0, c, P);
+        else k_probs_order<double><<<(unsigned)((c + 255) / 256), 256, 0, s->stream>>>((const double *)s->state, d_p, c0, c, P);
         k_chunk_totals<<<nblk, RB, 0, s->stream>>>(d_p, c, d_blk);
         k_chunk_offsets<<<1, 32, 0, s->stream>>>(d_blk, (int)nblk, d_carry);
+        QSB_CUDA(cudaGetLastError());
+        if (c0 + c <= first) continue;
         k_chunk_scan<<<nblk, RB, 0, s->stream>>>(d_p, c, d_blk);
         QSB_CUDA(cudaGetLastError());
-        QSB_CUDA(cudaMemcpyAsync(cdf + off, d_p, c * 8, cudaMemcpyDeviceToHost, s->stream));
+        const uint64_t skip = first > c0 ? first - c0 : 0;
+        QSB_CUDA(cudaMemcpyAsync(cdf + (c0 + skip - first), d_p + skip, (c - skip) * 8, cudaMemcpyDeviceToHost, s->stream));
         QSB_CUDA(cudaStreamSynchronize(s->stream));
     }
     return QSB_OK;

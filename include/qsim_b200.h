@@ -168,7 +168,12 @@ int qsb_norm_argmax(qsb_t *s, double *norm, uint64_t *argmax_idx, double *argmax
 int qsb_probabilities(qsb_t *s, double *p, uint64_t first, uint64_t count);
 /* Inclusive prefix sum of |a|^2 in logical index order -- compute_state_cumulative_distribution
  * (:256-268).  |a|^2 and the prefix sums are computed on the device (block scans chained by serial
- * offsets: monotone, equal to the reference's single fp64 accumulator up to re-association, <= 1e-12). */
+ * offsets: monotone, equal to the reference's single fp64 accumulator up to re-association, <= 1e-12).
+ * cdf[k] is the GLOBAL prefix sum at index first + k, i.e. it includes every |a_i|^2 with i < first:
+ * any range returns, bit for bit, the slice [first, first + count) of the full call (a range with
+ * first > 0 costs one extra read of the amplitudes below first).  One GPU only: on a sharded state it
+ * returns QSB_ERR_ARG, since the indices below a rank's own live on other ranks; qsb_sample draws
+ * shots from a sharded state. */
 int qsb_cdf(qsb_t *s, double *cdf, uint64_t first, uint64_t count);
 /* `shots` draws from the distribution; same search rule as measurement() (:270-283: first index
  * with cdf != 0 and cdf >= r, clamped to the last index), r from a seeded generator instead of

@@ -39,6 +39,11 @@ def check_sharded_readout(sim, got, n, rank, world, prec):
         assert p_phys[g_phys] > 0.0
         if g_phys != want:
             assert abs(cdf[want] - r) < 1e-9 or abs(cdf[g_phys] - r) < 1e-9, (k, r, g_phys, want)
+    try:                                   # the global CDF needs the other ranks' amplitudes: refused, not computed
+        sim.compute_state_cumulative_distribution(0, 1)
+        raise AssertionError("qsb_cdf accepted a sharded state")
+    except q.QsbError as e:
+        assert e.code == -1 and "qsb_sample" in str(e), e
     path = f"/tmp/qsb_shard_{os.getpid()}_{rank}.bin"
     before = sim.shard_physical().copy()
     sim.save_state(path)

@@ -31,16 +31,32 @@ def oracle_measure(cdf, n, r):
     return int(L.oc_measure(cdf.ctypes.data, n, r))
 
 
-def check_shots(shots, cdf, n, seed):
+def check_shots(shots, cdf, n, seed, rs=None):
     """Every shot is what the reference's search rule gives for the same r on the device CDF; a shot may only
-    differ when r sits within rounding of a CDF step."""
+    differ when r sits within rounding of a CDF step.  rs: the r of each shot, when the caller has them already
+    (q.sample_uniform replays the generator from shot 0, so a long run would cost time quadratic in its length)."""
     for k, got in enumerate(shots):
-        r = q.sample_uniform(seed, k)
+        r = q.sample_uniform(seed, k) if rs is None else float(rs[k])
         want = oracle_measure(cdf, n, r)
         if int(got) != want:
             assert abs(cdf[want] - r) < 1e-12 or abs(cdf[int(got)] - r) < 1e-12, (k, r, int(got), want)
         p = cdf[int(got)] - (cdf[int(got) - 1] if got else 0.0)
         assert p > 0.0
+
+
+def cdf_ranges(n, firsts=None):
+    """(first, count) pairs of qsb_cdf ranges that start off 0 (at 1, 255, 256 and just past the middle by default) and
+    end on a 4096-value block boundary, just past one, a few blocks on, or at the end."""
+    N = 1 << n
+    out = []
+    for first in firsts or (1, 255, 256, N // 2 + 3):
+        if first >= N:
+            continue
+        block_end = min(-(-(first + 1) // 4096) * 4096, N)
+        for end in sorted({first + 1, block_end, block_end + 1, first + 3 * 4096 + 17, N}):
+            if end <= N:
+                out.append((first, end - first))
+    return out
 
 
 @pytest.mark.parametrize("precision", [F32, F64], ids=["f32", "f64"])
@@ -58,6 +74,9 @@ def test_cdf_and_shots_after_a_fused_circuit(n, precision):
         assert abs(cdf[-1] - s.norm_argmax()[0]) < 1e-12
         part = s.compute_state_cumulative_distribution(first=0, count=(1 << n) // 2 + 1)
         assert np.array_equal(part, cdf[: (1 << n) // 2 + 1])
+        for first, count in cdf_ranges(n):                       # a range is the slice of the global CDF, bit for bit
+            part = s.compute_state_cumulative_distribution(first=first, count=count)
+            assert np.array_equal(part, cdf[first:first + count]), (first, count, part[0], cdf[first], cdf[first] - cdf[first - 1])
         shots = s.measurement(48, seed=11 + n)
         check_shots(shots, cdf, n, 11 + n)
         assert np.array_equal(shots, s.measurement(48, seed=11 + n))   # seeded: reproducible
