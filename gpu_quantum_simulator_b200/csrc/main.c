@@ -12,6 +12,9 @@
  *                       the reference keeps the state only in memory, quantum_simulator.c:75)
  *   --expect "Z0 Z1"    (repeatable) <psi|P|psi> of a Pauli string after the circuit, computed on the device:
  *                       one "EXPECTATION <text>: %.17g" line per flag, in flag order, after the --profile line
+ *   --marginal "0 3 5"  (repeatable) marginal probabilities of these qubits after the circuit, computed on the device:
+ *                       one "MARGINAL <qubits>: p_0 ... p_{2^k-1}" line (%.17g, bin b: bit i = value of the i-th
+ *                       qubit listed) per flag, in flag order, after the EXPECTATION lines
  *   --plan-only [--gpus N]   host-side fusion only (no GPU needed): one JSON line with the passes, rounds, ops and
  *                       qubit exchanges the circuit would run as on N ranks, instead of running it
  * Errors go to stdout followed by exit(1), like the reference (:56,:129,:213-219).
@@ -60,6 +63,7 @@ int main(int argc, char **argv)
     int precision = 32, dump = 0, shots = 0, prec_out = 0, profile = 0, sweep = 0, have_m = 0, plan_only = 0, gpus = 1;
     unsigned long long seed = 0; int have_seed = 0;
     const char **expect = (const char **)calloc((size_t)argc, sizeof(char *)); int n_expect = 0;
+    const char **marginal = (const char **)calloc((size_t)argc, sizeof(char *)); int n_marginal = 0;
     for (int i = 1; i < argc; i++) {
         if (!strcmp(argv[i], "--precision") && i + 1 < argc) precision = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--dump-amplitudes")) dump = 1;
@@ -74,6 +78,7 @@ int main(int argc, char **argv)
         else if (!strcmp(argv[i], "--gpus") && i + 1 < argc) gpus = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--sweep")) sweep = 1;
         else if (!strcmp(argv[i], "--expect") && i + 1 < argc) expect[n_expect++] = argv[++i];
+        else if (!strcmp(argv[i], "--marginal") && i + 1 < argc) marginal[n_marginal++] = argv[++i];
         else if (!file) file = argv[i];
         else if (!have_m) { num_m = atol(argv[i]); have_m = 1; }
     }
@@ -131,6 +136,30 @@ int main(int argc, char **argv)
         for (int k = 0; k < n_expect; k++) printf("EXPECTATION %s: %.17g\n", expect[k], ev[k]);
         free(ex); free(ev);
     }
+    for (int m = 0; m < n_marginal; m++) {   /* "0 3 5": whitespace-separated qubits */
+        int qs[64], k = 0;
+        const char *p = marginal[m];
+        for (;;) {
+            while (*p == ' ' || *p == '\t') p++;
+            if (!*p) break;
+            char *end;
+            long v = strtol(p, &end, 10);
+            if (end == p || (*end && *end != ' ' && *end != '\t') || v < 0 || v > 1000000 || k == 64) {
+                printf("--marginal \"%s\": expected a whitespace-separated list of qubits\n", marginal[m]); return 1;
+            }
+            qs[k++] = (int)v;
+            p = end;
+        }
+        double *mp = (double *)malloc(sizeof(double) * ((size_t)1 << (k < 20 ? k : 20)));
+        if (!mp) { printf("Malloc error\n"); return 1; }
+        if (qsb_marginal_probabilities(s, qs, k, mp)) { printf("%s\n", qsb_last_error()); return 1; }
+        printf("MARGINAL");
+        for (int i = 0; i < k; i++) printf(" %d", qs[i]);
+        printf(":");
+        for (size_t b = 0; b < ((size_t)1 << k); b++) printf(" %.17g", mp[b]);
+        printf("\n");
+        free(mp);
+    }
     const unsigned long long N = 1ULL << nq;
     if (dump || dump_bin) {
         const unsigned long long chunk = 1ULL << 20;
@@ -169,5 +198,6 @@ int main(int argc, char **argv)
     qsb_destroy(s);
     qsb_free(gates);
     free(expect);
+    free(marginal);
     return 0;
 }

@@ -290,6 +290,45 @@ class Simulator:
         check(lib.qsb_expectation_pauli(self._h, x.ctypes.data, z.ctypes.data, x.size, out.ctypes.data))
         return float(out[0]) if isinstance(paulis, str) else out
 
+    # ---- marginals and projective measurement (bit i of a bin index or an outcome is the value of qubits[i])
+    @staticmethod
+    def _qubits(qubits):
+        return np.ascontiguousarray(np.asarray(qubits, dtype=np.int32).reshape(-1))
+
+    def marginal_probabilities(self, qubits):
+        """float64 array of 2^k values: entry b is the probability that qubits[i] reads bit i of b for every i, so
+        [3, 0] gives the transposed table of [0, 3].  Computed on the device in one read of the state; the state and
+        the qubit layout are left as they are, nothing is renormalised.  1 <= k <= min(n, 20)."""
+        qs = self._qubits(qubits)
+        out = np.empty(1 << min(qs.size, 20), dtype=np.float64)
+        check(lib.qsb_marginal_probabilities(self._h, qs.ctypes.data, qs.size, out.ctypes.data))
+        return out
+
+    def collapse(self, qubits, outcome):
+        """Project onto `outcome` (bit i = value of qubits[i]) and rescale to norm 1; returns its probability p,
+        equal bit for bit to marginal_probabilities(qubits)[outcome].  p == 0 is refused and leaves the state as it is."""
+        qs = self._qubits(qubits)
+        p = C.c_double()
+        check(lib.qsb_collapse(self._h, qs.ctypes.data, qs.size, int(outcome), C.byref(p)))
+        return p.value
+
+    def measure_qubits(self, qubits, r):
+        """Measure these qubits with the uniform number r in [0, 1) (e.g. sample_uniform(seed, k)) and collapse the
+        state onto the outcome; returns (outcome, p), bit i of the outcome = value of qubits[i].  The outcome is the
+        first bin whose inclusive prefix sum C_b of the marginal table is != 0 and >= r * total."""
+        qs = self._qubits(qubits)
+        b, p = C.c_uint64(), C.c_double()
+        check(lib.qsb_measure_qubits(self._h, qs.ctypes.data, qs.size, float(r), C.byref(b), C.byref(p)))
+        return b.value, p.value
+
+    def reset_qubits(self, qubits, r):
+        """measure_qubits, then X on every qubit that came out 1, so the qubits end in |0>; returns the outcome
+        (bit i = value qubits[i] had)."""
+        qs = self._qubits(qubits)
+        b = C.c_uint64()
+        check(lib.qsb_reset_qubits(self._h, qs.ctypes.data, qs.size, float(r), C.byref(b)))
+        return b.value
+
     def save_state(self, path):
         """Dump this rank's shard (device dtype, physical order) with its qubit map; one file per rank."""
         check(lib.qsb_save_state(self._h, os.fsencode(path)))

@@ -211,6 +211,35 @@ int qsb_pauli_from_string(const char *text, int num_qubits, uint64_t *x, uint64_
 int qsb_expectation_dry_run(int num_qubits, const qsb_options_t *opt, const uint64_t *x, const uint64_t *z,
                             size_t nterms, uint32_t *sweeps, uint32_t *exchanges);
 
+/* ---- marginals and projective measurement ----------------------------------
+ * The measured qubits are an array qubits[0..k-1] of distinct LOGICAL qubits, 1 <= k <= min(n, 20).  Bit i of a bin
+ * index or an outcome is the value of qubits[i], so {3, 0} gives the transposed table of {0, 3}.  All sums are fp64
+ * over the state as stored; nothing is renormalised.  More than 20 qubits are measured in groups: measuring disjoint
+ * groups one after another gives the same joint distribution (the Born rule chain p(a) p(b | a)).
+ * Errors return QSB_ERR_ARG and leave the state untouched: a repeated qubit, a qubit outside [0, n), k outside
+ * [1, min(n, 20)], a null pointer (other than the optional prob / outcome noted below), an outcome >= 2^k.  On a
+ * sharded state these calls are collective (same arguments on every rank) and need qsb_comm_init (else QSB_ERR_COMM);
+ * every rank receives the same values, bit for bit. */
+/* out[b] = sum of |a_j|^2 over every j whose bits qubits[i] equal bit i of b; 2^k values.  One read of the local shard.
+ * Deterministic: repeated calls return identical bits.  Does not change the state or the qubit layout. */
+int qsb_marginal_probabilities(qsb_t *s, const int *qubits, int k, double *out);
+/* Project onto outcome `outcome` of these qubits and scale the kept amplitudes by 1/sqrt(p), p = the marginal of that
+ * outcome (equal bit for bit to its qsb_marginal_probabilities entry), so the state has norm 1.  *prob = p (prob may
+ * be NULL).  p == 0 -> QSB_ERR_ARG and the state is unchanged.  The qubit layout is unchanged.  Cost: a read of the
+ * kept amplitudes for p, then one pass that writes the shard and reads only the kept amplitudes. */
+int qsb_collapse(qsb_t *s, const int *qubits, int k, uint64_t outcome, double *prob);
+/* The marginal table, then the outcome by the rule of measurement() (quantum_simulator.c:279) on that table: the first
+ * b with C_b != 0 and C_b >= r * T, where C_b is the inclusive serial fp64 prefix sum of the table in bin order and
+ * T = C_{2^k - 1}; then the collapse onto it (*prob = its table entry; prob may be NULL).  r in [0, 1), e.g. from
+ * qsb_sample_uniform.  T == 0, or r outside [0, 1) or NaN -> QSB_ERR_ARG, state unchanged.  With r < 1 and T > 0 the
+ * rule always picks a bin with p > 0 (C_b >= r * T is reached at the latest by the last bin, and a bin with p = 0
+ * repeats the C of the bin before it), so there is no clamp case.  Sharded: the same r on every rank gives every rank
+ * the same outcome. */
+int qsb_measure_qubits(qsb_t *s, const int *qubits, int k, double r, uint64_t *outcome, double *prob);
+/* qsb_measure_qubits, then X (through qsb_apply_gates) on every measured qubit that came out 1: the qubits end in |0>.
+ * *outcome = the measured outcome (outcome may be NULL). */
+int qsb_reset_qubits(qsb_t *s, const int *qubits, int k, double r, uint64_t *outcome);
+
 /* ---- shard dump / reload ----------------------------------------------------
  * The reference keeps the state only in memory (quantum_simulator.c:75 frees it
  * at exit); long sharded runs want a checkpoint.  File = 128-byte header (magic
