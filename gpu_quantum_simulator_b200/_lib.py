@@ -71,6 +71,7 @@ SYMBOLS = {
     "qsb_measure_qubits": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.POINTER(C.c_uint64),
                                      C.POINTER(C.c_double)]),
     "qsb_reset_qubits": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.POINTER(C.c_uint64)]),
+    "qsb_reduced_density_matrix": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "qsb_save_state": (C.c_int, [C.c_void_p, C.c_char_p]),
     "qsb_load_state": (C.c_int, [C.c_void_p, C.c_char_p]),
     "qsb_comm_unique_id": (C.c_int, [C.c_void_p]),

@@ -15,6 +15,9 @@
  *   --marginal "0 3 5"  (repeatable) marginal probabilities of these qubits after the circuit, computed on the device:
  *                       one "MARGINAL <qubits>: p_0 ... p_{2^k-1}" line (%.17g, bin b: bit i = value of the i-th
  *                       qubit listed) per flag, in flag order, after the EXPECTATION lines
+ *   --rdm "0 3"         (repeatable) reduced density matrix of these qubits after the circuit, computed on the device:
+ *                       one "RDM <qubits>: re_00 im_00 re_01 im_01 ..." line (%.17g, row-major, row / column index: bit i
+ *                       = value of the i-th qubit listed) per flag, in flag order, after the MARGINAL lines
  *   --plan-only [--gpus N]   host-side fusion only (no GPU needed): one JSON line with the passes, rounds, ops and
  *                       qubit exchanges the circuit would run as on N ranks, instead of running it
  * Errors go to stdout followed by exit(1), like the reference (:56,:129,:213-219).
@@ -56,6 +59,22 @@ static void format_help(void)
     printf("(extensions: y p rx ry u cz cy ch cp swap ccx, gate definitions, ctrl/negctrl/inv/pow modifiers, gphase, pi expressions)\n");
 }
 
+/* "0 3 5": whitespace-separated qubits -> qs[0..*k-1]; 0 when the text is not such a list */
+static int parse_qubits(const char *text, int qs[64], int *k)
+{
+    const char *p = text;
+    *k = 0;
+    for (;;) {
+        while (*p == ' ' || *p == '\t') p++;
+        if (!*p) return 1;
+        char *end;
+        long v = strtol(p, &end, 10);
+        if (end == p || (*end && *end != ' ' && *end != '\t') || v < 0 || v > 1000000 || *k == 64) return 0;
+        qs[(*k)++] = (int)v;
+        p = end;
+    }
+}
+
 int main(int argc, char **argv)
 {
     const char *file = NULL, *dump_bin = NULL, *save_state = NULL, *load_state = NULL;
@@ -64,6 +83,7 @@ int main(int argc, char **argv)
     unsigned long long seed = 0; int have_seed = 0;
     const char **expect = (const char **)calloc((size_t)argc, sizeof(char *)); int n_expect = 0;
     const char **marginal = (const char **)calloc((size_t)argc, sizeof(char *)); int n_marginal = 0;
+    const char **rdm = (const char **)calloc((size_t)argc, sizeof(char *)); int n_rdm = 0;
     for (int i = 1; i < argc; i++) {
         if (!strcmp(argv[i], "--precision") && i + 1 < argc) precision = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--dump-amplitudes")) dump = 1;
@@ -79,6 +99,7 @@ int main(int argc, char **argv)
         else if (!strcmp(argv[i], "--sweep")) sweep = 1;
         else if (!strcmp(argv[i], "--expect") && i + 1 < argc) expect[n_expect++] = argv[++i];
         else if (!strcmp(argv[i], "--marginal") && i + 1 < argc) marginal[n_marginal++] = argv[++i];
+        else if (!strcmp(argv[i], "--rdm") && i + 1 < argc) rdm[n_rdm++] = argv[++i];
         else if (!file) file = argv[i];
         else if (!have_m) { num_m = atol(argv[i]); have_m = 1; }
     }
@@ -136,19 +157,10 @@ int main(int argc, char **argv)
         for (int k = 0; k < n_expect; k++) printf("EXPECTATION %s: %.17g\n", expect[k], ev[k]);
         free(ex); free(ev);
     }
-    for (int m = 0; m < n_marginal; m++) {   /* "0 3 5": whitespace-separated qubits */
+    for (int m = 0; m < n_marginal; m++) {
         int qs[64], k = 0;
-        const char *p = marginal[m];
-        for (;;) {
-            while (*p == ' ' || *p == '\t') p++;
-            if (!*p) break;
-            char *end;
-            long v = strtol(p, &end, 10);
-            if (end == p || (*end && *end != ' ' && *end != '\t') || v < 0 || v > 1000000 || k == 64) {
-                printf("--marginal \"%s\": expected a whitespace-separated list of qubits\n", marginal[m]); return 1;
-            }
-            qs[k++] = (int)v;
-            p = end;
+        if (!parse_qubits(marginal[m], qs, &k)) {
+            printf("--marginal \"%s\": expected a whitespace-separated list of qubits\n", marginal[m]); return 1;
         }
         double *mp = (double *)malloc(sizeof(double) * ((size_t)1 << (k < 20 ? k : 20)));
         if (!mp) { printf("Malloc error\n"); return 1; }
@@ -159,6 +171,22 @@ int main(int argc, char **argv)
         for (size_t b = 0; b < ((size_t)1 << k); b++) printf(" %.17g", mp[b]);
         printf("\n");
         free(mp);
+    }
+    for (int m = 0; m < n_rdm; m++) {
+        int qs[64], k = 0;
+        if (!parse_qubits(rdm[m], qs, &k)) {
+            printf("--rdm \"%s\": expected a whitespace-separated list of qubits\n", rdm[m]); return 1;
+        }
+        const size_t d = (size_t)1 << (k < 12 ? k : 12);   /* a larger k is refused before anything is written */
+        double *rho = (double *)malloc(sizeof(double) * 2 * d * d);
+        if (!rho) { printf("Malloc error\n"); return 1; }
+        if (qsb_reduced_density_matrix(s, qs, k, rho)) { printf("%s\n", qsb_last_error()); return 1; }
+        printf("RDM");
+        for (int i = 0; i < k; i++) printf(" %d", qs[i]);
+        printf(":");
+        for (size_t e = 0; e < 2 * d * d; e++) printf(" %.17g", rho[e]);
+        printf("\n");
+        free(rho);
     }
     const unsigned long long N = 1ULL << nq;
     if (dump || dump_bin) {
@@ -199,5 +227,6 @@ int main(int argc, char **argv)
     qsb_free(gates);
     free(expect);
     free(marginal);
+    free(rdm);
     return 0;
 }

@@ -47,6 +47,7 @@ int tiled_comm_allgather(qsb_sim *s, const void *dsrc, void *ddst, size_t bytes)
 #define MRG_NU 16                    /* units (16 bytes) per thread and tile, at most */
 #define MRG_UB 4                     /* log2(MRG_NU) */
 #define MRG_KMAX 20                  /* qubits per call */
+#define MRG_HINT "measure more than 20 qubits in groups"
 #define MRG_TABLE_BYTES ((size_t)8 << 20)   /* 2^20 fp64 bins at the start of the staging buffer */
 #define MRG_CTA_TARGET_LOG2 13       /* ~8192 CTAs: many waves of 148 SMs, a small tail */
 /* the in-tile bits (pack + thread bits) exist in every shard: nloc >= tiled_min_local_bits() */
@@ -187,6 +188,25 @@ __global__ void __launch_bounds__(256) k_collapse(uint4 *A, uint64_t nunits, uin
 
 /* ================================================================================================ host */
 
+/* the argument rules shared by the calls that take a list of qubits (measure.cu, rdm.cu) */
+int check_qubits(const qsb_sim *s, const int *qubits, int k, int kmax, const char *fn, const char *hint)
+{
+    if (!qubits) { qsb_set_error("%s: null qubit array", fn); return QSB_ERR_ARG; }
+    kmax = std::min(s->n, kmax);
+    if (k < 1 || k > kmax) {
+        qsb_set_error("%s: %d qubits, expected 1..%d (%s)", fn, k, kmax, hint);
+        return QSB_ERR_ARG;
+    }
+    uint64_t seen = 0;
+    for (int i = 0; i < k; i++) {
+        const int q = qubits[i];
+        if (q < 0 || q >= s->n) { qsb_set_error("%s: qubit %d outside [0, %d)", fn, q, s->n); return QSB_ERR_ARG; }
+        if ((seen >> q) & 1) { qsb_set_error("%s: qubit %d appears twice", fn, q); return QSB_ERR_ARG; }
+        seen |= 1ULL << q;
+    }
+    return QSB_OK;
+}
+
 namespace {
 
 struct Geom {
@@ -199,24 +219,6 @@ struct Geom {
     std::vector<int> lq, rq;           /* indices i into qubits[] on local / rank bits, in qubits[] order */
     std::vector<int> lphys, rbit;      /* their physical bit / rank bit */
 };
-
-int check_qubits(const qsb_sim *s, const int *qubits, int k, const char *fn)
-{
-    if (!qubits) { qsb_set_error("%s: null qubit array", fn); return QSB_ERR_ARG; }
-    const int kmax = std::min(s->n, MRG_KMAX);
-    if (k < 1 || k > kmax) {
-        qsb_set_error("%s: %d qubits, expected 1..%d (measure more than %d qubits in groups)", fn, k, kmax, MRG_KMAX);
-        return QSB_ERR_ARG;
-    }
-    uint64_t seen = 0;
-    for (int i = 0; i < k; i++) {
-        const int q = qubits[i];
-        if (q < 0 || q >= s->n) { qsb_set_error("%s: qubit %d outside [0, %d)", fn, q, s->n); return QSB_ERR_ARG; }
-        if ((seen >> q) & 1) { qsb_set_error("%s: qubit %d appears twice", fn, q); return QSB_ERR_ARG; }
-        seen |= 1ULL << q;
-    }
-    return QSB_OK;
-}
 
 void geometry(const qsb_sim *s, const int *qubits, int k, Geom &G)
 {
@@ -420,7 +422,7 @@ int pick_outcome(const std::vector<double> &tab, double r, uint64_t *b_out, cons
 int measure_common(qsb_sim *s, const int *qubits, int k, double r, uint64_t *outcome, double *prob, const char *fn)
 {
     if (!s) { qsb_set_error("%s: null handle", fn); return QSB_ERR_ARG; }
-    int rc = check_qubits(s, qubits, k, fn);
+    int rc = check_qubits(s, qubits, k, MRG_KMAX, fn, MRG_HINT);
     if (rc) return rc;
     if (!outcome) { qsb_set_error("%s: null outcome", fn); return QSB_ERR_ARG; }
     if (!(r >= 0.0 && r < 1.0)) { qsb_set_error("%s: r = %g outside [0, 1)", fn, r); return QSB_ERR_ARG; }
@@ -448,7 +450,7 @@ int measure_common(qsb_sim *s, const int *qubits, int k, double r, uint64_t *out
 extern "C" int qsb_marginal_probabilities(qsb_t *s, const int *qubits, int k, double *out)
 {
     if (!s) { qsb_set_error("qsb_marginal_probabilities: null handle"); return QSB_ERR_ARG; }
-    int rc = check_qubits(s, qubits, k, "qsb_marginal_probabilities");
+    int rc = check_qubits(s, qubits, k, MRG_KMAX, "qsb_marginal_probabilities", MRG_HINT);
     if (rc) return rc;
     if (!out) { qsb_set_error("qsb_marginal_probabilities: null output"); return QSB_ERR_ARG; }
     if (s->g && !s->comm) { qsb_set_error("qsb_marginal_probabilities: sharded state needs qsb_comm_init first"); return QSB_ERR_COMM; }
@@ -461,7 +463,7 @@ extern "C" int qsb_marginal_probabilities(qsb_t *s, const int *qubits, int k, do
 extern "C" int qsb_collapse(qsb_t *s, const int *qubits, int k, uint64_t outcome, double *prob)
 {
     if (!s) { qsb_set_error("qsb_collapse: null handle"); return QSB_ERR_ARG; }
-    int rc = check_qubits(s, qubits, k, "qsb_collapse");
+    int rc = check_qubits(s, qubits, k, MRG_KMAX, "qsb_collapse", MRG_HINT);
     if (rc) return rc;
     if (outcome >> k) { qsb_set_error("qsb_collapse: outcome %llu >= 2^%d", (unsigned long long)outcome, k); return QSB_ERR_ARG; }
     if (s->g && !s->comm) { qsb_set_error("qsb_collapse: sharded state needs qsb_comm_init first"); return QSB_ERR_COMM; }

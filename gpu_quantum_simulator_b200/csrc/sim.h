@@ -53,5 +53,9 @@ struct qsb_plan {
 /* canonicalise source gates -> COps (+ global phase) */
 int qsb_canonicalise(const qsb_gate_t *gates, size_t n, int num_qubits, std::vector<COp> &out, double gphase[2]);
 
+/* QSB_ERR_ARG (with a message naming fn) unless qubits[0..k-1] are distinct qubits of the handle and 1 <= k <=
+ * min(n, kmax); hint says what to do about a k above kmax */
+int check_qubits(const qsb_sim *s, const int *qubits, int k, int kmax, const char *fn, const char *hint);
+
 /* element size of one amplitude */
 static inline size_t amp_bytes(int prec) { return prec == QSB_F64 ? 16 : 8; }

@@ -329,6 +329,29 @@ class Simulator:
         check(lib.qsb_reset_qubits(self._h, qs.ctypes.data, qs.size, float(r), C.byref(b)))
         return b.value
 
+    # ---- reduced density matrices (bit i of a row or column index is the value of qubits[i])
+    def reduced_density_matrix(self, qubits):
+        """complex128 array of shape (2^k, 2^k): rho[a, b] = sum of a_j conj(a_j') over the index pairs that agree on every
+        other qubit and read a / b on `qubits`, i.e. the partial trace of |psi><psi| over the other qubits.  Computed on
+        the device in fp64 on the state as stored (trace = the norm, nothing is renormalised), exactly Hermitian, bit
+        for bit the same on repeat; the state and the qubit layout are left as they are.  1 <= k <= min(n, 12)."""
+        qs = self._qubits(qubits)
+        d = 1 << min(qs.size, 12)              # larger k is refused by the library before it writes
+        out = np.empty(2 * d * d, dtype=np.float64)
+        check(lib.qsb_reduced_density_matrix(self._h, qs.ctypes.data, qs.size, out.ctypes.data))
+        return out.view(np.complex128).reshape(d, d)
+
+    def entanglement_entropy(self, qubits, base=2):
+        """von Neumann entropy -sum w log w of rho / Tr rho for rho = reduced_density_matrix(qubits), from the
+        eigenvalues w of np.linalg.eigvalsh on the host; eigenvalues <= 0 count as 0."""
+        rho = self.reduced_density_matrix(qubits)
+        tr = float(np.trace(rho).real)
+        if not tr > 0.0:
+            raise ValueError(f"the state has norm {tr}: no entropy")
+        w = np.linalg.eigvalsh(rho / tr)
+        w = w[w > 0.0]
+        return float(-np.sum(w * np.log(w)) / np.log(base))
+
     def save_state(self, path):
         """Dump this rank's shard (device dtype, physical order) with its qubit map; one file per rank."""
         check(lib.qsb_save_state(self._h, os.fsencode(path)))

@@ -240,6 +240,29 @@ int qsb_measure_qubits(qsb_t *s, const int *qubits, int k, double r, uint64_t *o
  * *outcome = the measured outcome (outcome may be NULL). */
 int qsb_reset_qubits(qsb_t *s, const int *qubits, int k, double r, uint64_t *outcome);
 
+/* ---- reduced density matrices ------------------------------------------------
+ * rho = Tr_{other qubits} |psi><psi| for qubits[0..k-1], 1 <= k <= min(n, 12), with the qubit conventions and argument
+ * rules of the marginals above: distinct LOGICAL qubits, bit i of a and b is the value of qubits[i], so {3, 0} gives the
+ * matrix of {0, 3} with its indices re-ordered.  rho has 2 * 4^k doubles: entry (a, b) at rho[2 * (a * 2^k + b)] (re)
+ * and [.. + 1] (im):
+ *     rho[a][b] = sum over j, j' that agree on every other qubit, with bits(j) = a and bits(j') = b, of a_j * conj(a_j')
+ * Everything is fp64 on the state as stored, with no renormalisation: Tr rho = the norm, and the diagonal is the
+ * qsb_marginal_probabilities table up to the order of the additions.  Exactly Hermitian: only the entries with a <= b
+ * are computed and the others are their mirror, so rho[b][a] == conj(rho[a][b]) bit for bit and every diagonal imaginary
+ * part is +0.0.  Deterministic: reductions run in a fixed order, repeated calls return identical bits.  Does not change
+ * the state, the qubit layout, the role of the exchange buffer or the peer mappings.
+ * Errors return QSB_ERR_ARG and leave the state untouched: a null handle, qubit array or rho, k outside [1, min(n, 12)],
+ * a repeated qubit, a qubit outside [0, n).  A sharded handle without qsb_comm_init gives QSB_ERR_COMM.  The device
+ * scratch is one allocation per call, freed before it returns (QSB_ERR_NOMEM if it fails): 2^m 4^(k - m) x 16 bytes for
+ * the local matrices (m = measured qubits on rank bits), at most 64 MiB of per-block partials, and on a sharded state
+ * world times the local matrices for their all-gather (host memory holds the same); at k = 12 on one GPU that is 256 MiB
+ * plus the partials, on 8 ranks with no rank qubit measured 2.25 GiB.
+ * Cost: one read of the local shard for 2^k_loc <= 64 (k_loc = measured qubits on local bits), about 2^k_loc / 64 reads
+ * above, and 4 * 2^n_loc * (2^k_loc + 1) fp64 flops.  On a sharded state the call is collective (same arguments on every
+ * rank), each rank receives the shard of a partner rank into its exchange buffer once per non-zero pattern of the
+ * measured rank qubits (2^m - 1 shard copies per call), and every rank receives the same bits. */
+int qsb_reduced_density_matrix(qsb_t *s, const int *qubits, int k, double *rho);
+
 /* ---- shard dump / reload ----------------------------------------------------
  * The reference keeps the state only in memory (quantum_simulator.c:75 frees it
  * at exit); long sharded runs want a checkpoint.  File = 128-byte header (magic
