@@ -39,6 +39,7 @@
 #include <map>
 #include <vector>
 
+#include "pauli.h"
 #include "sim.h"
 #include "tiled.h"
 
@@ -207,19 +208,6 @@ __global__ void k_expect_finish(const double *partial, int nblk, int K, const Ex
 
 /* ================================================================================================ host */
 
-namespace {
-
-struct PhysTerm { uint64_t xl, zl, xr, zr; int y; };   /* local / rank-bit parts of the physical masks */
-
-struct ExpSweep {
-    uint64_t xr = 0;               /* rank-bit flips: partner rank = rank ^ xr */
-    int8_t pb[16];                 /* tile coordinate bit j -> local physical bit */
-    uint64_t bmask = 0, x_out = 0; /* tile bits, local flips outside the tile */
-    std::vector<uint32_t> terms;
-};
-
-inline int parity64(uint64_t v) { return __builtin_popcountll(v) & 1; }
-
 int exp_geometry(int prec, const qsb_options_t *opt, int *T, int *L)
 {
     *T = prec == QSB_F64 ? EXP_T_F64 : EXP_T_F32;
@@ -228,6 +216,64 @@ int exp_geometry(int prec, const qsb_options_t *opt, int *T, int *L)
     *L = std::min(l, *T);
     return QSB_OK;
 }
+
+int check_terms(int n, const uint64_t *x, const uint64_t *z, size_t nterms, const char *fn)
+{
+    if (nterms && (!x || !z)) { qsb_set_error("%s: null term array", fn); return QSB_ERR_ARG; }
+    const uint64_t bad = n >= 64 ? 0 : ~((1ULL << n) - 1);
+    for (size_t i = 0; i < nterms; i++)
+        if ((x[i] | z[i]) & bad) {
+            qsb_set_error("%s: term %zu has a qubit >= %d (x = 0x%llx, z = 0x%llx)", fn, i, n, (unsigned long long)x[i], (unsigned long long)z[i]);
+            return QSB_ERR_ARG;
+        }
+    return QSB_OK;
+}
+
+void to_physical(int n, int nloc, const BitPerm &perm, const uint64_t *x, const uint64_t *z, size_t nterms, std::vector<PhysTerm> &out)
+{
+    out.resize(nterms);
+    for (size_t i = 0; i < nterms; i++) {
+        uint64_t px = 0, pz = 0;
+        for (int q = 0; q < n; q++) {
+            if ((x[i] >> q) & 1) px |= 1ULL << perm.pos[q];
+            if ((z[i] >> q) & 1) pz |= 1ULL << perm.pos[q];
+        }
+        const uint64_t loc = (1ULL << nloc) - 1;
+        out[i] = PhysTerm{px & loc, pz & loc, px >> nloc, pz >> nloc, __builtin_popcountll(x[i] & z[i]) & 3};
+    }
+}
+
+uint32_t tile_coord(uint64_t m, const int8_t *pb, int T)
+{
+    uint32_t r = 0;
+    for (int j = 0; j < T; j++) r |= (uint32_t)((m >> pb[j]) & 1) << j;
+    return r;
+}
+
+static int ilog2i(int v) { int r = 0; while ((1 << r) < v) r++; return r; }
+
+int pauli_dry_run_shape(int num_qubits, const qsb_options_t *opt_in, qsb_options_t *opt, int *nloc)
+{
+    if (num_qubits < 1 || num_qubits > 40) { qsb_set_error("num_qubits %d out of range 1..40", num_qubits); return QSB_ERR_ARG; }
+    if (opt_in) *opt = *opt_in; else qsb_options_default(opt);
+    if (opt->precision == 0) opt->precision = QSB_F32;
+    if (opt->precision != QSB_F32 && opt->precision != QSB_F64) { qsb_set_error("precision must be 32 or 64"); return QSB_ERR_ARG; }
+    if (opt->world_size <= 0) opt->world_size = 1;
+    if (opt->world_size & (opt->world_size - 1)) { qsb_set_error("world_size must be a power of two"); return QSB_ERR_ARG; }
+    const int g = ilog2i(opt->world_size), min_loc = tiled_min_local_bits(opt->precision, opt);
+    if (g > 0 && num_qubits - g < min_loc + g) { qsb_set_error("%d qubits are too few to shard over %d ranks", num_qubits, opt->world_size); return QSB_ERR_ARG; }
+    *nloc = std::max(num_qubits - g, min_loc);
+    return QSB_OK;
+}
+
+namespace {
+
+struct ExpSweep {
+    uint64_t xr = 0;               /* rank-bit flips: partner rank = rank ^ xr */
+    int8_t pb[16];                 /* tile coordinate bit j -> local physical bit */
+    uint64_t bmask = 0, x_out = 0; /* tile bits, local flips outside the tile */
+    std::vector<uint32_t> terms;
+};
 
 /* Greedy cover of the distinct physical x masks by sweeps (host only, no CUDA).  Sweeps come grouped by xr,
  * xr == 0 first, so that each partner shard is fetched once. */
@@ -295,40 +341,6 @@ uint32_t count_exchanges(const std::vector<ExpSweep> &sw)
     return n;
 }
 
-int check_terms(int n, const uint64_t *x, const uint64_t *z, size_t nterms, const char *fn)
-{
-    if (nterms && (!x || !z)) { qsb_set_error("%s: null term array", fn); return QSB_ERR_ARG; }
-    const uint64_t bad = n >= 64 ? 0 : ~((1ULL << n) - 1);
-    for (size_t i = 0; i < nterms; i++)
-        if ((x[i] | z[i]) & bad) {
-            qsb_set_error("%s: term %zu has a qubit >= %d (x = 0x%llx, z = 0x%llx)", fn, i, n, (unsigned long long)x[i], (unsigned long long)z[i]);
-            return QSB_ERR_ARG;
-        }
-    return QSB_OK;
-}
-
-void to_physical(int n, int nloc, const BitPerm &perm, const uint64_t *x, const uint64_t *z, size_t nterms, std::vector<PhysTerm> &out)
-{
-    out.resize(nterms);
-    for (size_t i = 0; i < nterms; i++) {
-        uint64_t px = 0, pz = 0;
-        for (int q = 0; q < n; q++) {
-            if ((x[i] >> q) & 1) px |= 1ULL << perm.pos[q];
-            if ((z[i] >> q) & 1) pz |= 1ULL << perm.pos[q];
-        }
-        const uint64_t loc = (1ULL << nloc) - 1;
-        out[i] = PhysTerm{px & loc, pz & loc, px >> nloc, pz >> nloc, __builtin_popcountll(x[i] & z[i]) & 3};
-    }
-}
-
-/* compress the bits of m at the positions pb[0..T-1] */
-uint32_t tile_coord(uint64_t m, const int8_t *pb, int T)
-{
-    uint32_t r = 0;
-    for (int j = 0; j < T; j++) r |= (uint32_t)((m >> pb[j]) & 1) << j;
-    return r;
-}
-
 ExpTerm encode_term(const PhysTerm &p, const ExpSweep &sw, bool f32, uint32_t out_index)
 {
     const int T = f32 ? EXP_T_F32 : EXP_T_F64, s = f32 ? 1 : 0;   /* s: unit-address shift (f32 units hold two amplitudes) */
@@ -384,23 +396,15 @@ extern "C" int qsb_pauli_from_string(const char *text, int num_qubits, uint64_t 
     return QSB_OK;
 }
 
-static int ilog2i(int v) { int r = 0; while ((1 << r) < v) r++; return r; }
-
 extern "C" int qsb_expectation_dry_run(int num_qubits, const qsb_options_t *opt_in, const uint64_t *x, const uint64_t *z,
                                        size_t nterms, uint32_t *sweeps, uint32_t *exchanges)
 {
-    if (num_qubits < 1 || num_qubits > 40) { qsb_set_error("num_qubits %d out of range 1..40", num_qubits); return QSB_ERR_ARG; }
     qsb_options_t opt;
-    if (opt_in) opt = *opt_in; else qsb_options_default(&opt);
-    if (opt.precision == 0) opt.precision = QSB_F32;
-    if (opt.precision != QSB_F32 && opt.precision != QSB_F64) { qsb_set_error("precision must be 32 or 64"); return QSB_ERR_ARG; }
-    if (opt.world_size <= 0) opt.world_size = 1;
-    if (opt.world_size & (opt.world_size - 1)) { qsb_set_error("world_size must be a power of two"); return QSB_ERR_ARG; }
-    int rc = check_terms(num_qubits, x, z, nterms, "qsb_expectation_dry_run");
+    int nloc;
+    int rc = pauli_dry_run_shape(num_qubits, opt_in, &opt, &nloc);
     if (rc) return rc;
-    const int g = ilog2i(opt.world_size), min_loc = tiled_min_local_bits(opt.precision, &opt);
-    if (g > 0 && num_qubits - g < min_loc + g) { qsb_set_error("%d qubits are too few to shard over %d ranks", num_qubits, opt.world_size); return QSB_ERR_ARG; }
-    const int nloc = std::max(num_qubits - g, min_loc);
+    rc = check_terms(num_qubits, x, z, nterms, "qsb_expectation_dry_run");
+    if (rc) return rc;
     BitPerm id; for (int q = 0; q < 64; q++) id.pos[q] = (int8_t)q;
     int T, L;
     exp_geometry(opt.precision, &opt, &T, &L);

@@ -10,6 +10,8 @@
  *   <number_of_measurement> > 0 with --shots: "MEASUREMENT: <bits> (%ld)" (quantum_simulator.c:68-73)
  *   --save-state FILE / --load-state FILE   raw shard + qubit map after / before the circuit (checkpoint;
  *                       the reference keeps the state only in memory, quantum_simulator.c:75)
+ *   --pauli-rot "X0 Z3" 0.25   (repeatable) the rotation exp(-i 0.25 P / 2) applied on the device after the circuit (after
+ *                       --load-state, before --save-state), in flag order, so the lines below read the rotated state
  *   --expect "Z0 Z1"    (repeatable) <psi|P|psi> of a Pauli string after the circuit, computed on the device:
  *                       one "EXPECTATION <text>: %.17g" line per flag, in flag order, after the --profile line
  *   --marginal "0 3 5"  (repeatable) marginal probabilities of these qubits after the circuit, computed on the device:
@@ -84,6 +86,8 @@ int main(int argc, char **argv)
     const char **expect = (const char **)calloc((size_t)argc, sizeof(char *)); int n_expect = 0;
     const char **marginal = (const char **)calloc((size_t)argc, sizeof(char *)); int n_marginal = 0;
     const char **rdm = (const char **)calloc((size_t)argc, sizeof(char *)); int n_rdm = 0;
+    const char **rot = (const char **)calloc((size_t)argc, sizeof(char *)); int n_rot = 0;
+    double *rot_theta = (double *)calloc((size_t)argc, sizeof(double));
     for (int i = 1; i < argc; i++) {
         if (!strcmp(argv[i], "--precision") && i + 1 < argc) precision = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--dump-amplitudes")) dump = 1;
@@ -100,6 +104,13 @@ int main(int argc, char **argv)
         else if (!strcmp(argv[i], "--expect") && i + 1 < argc) expect[n_expect++] = argv[++i];
         else if (!strcmp(argv[i], "--marginal") && i + 1 < argc) marginal[n_marginal++] = argv[++i];
         else if (!strcmp(argv[i], "--rdm") && i + 1 < argc) rdm[n_rdm++] = argv[++i];
+        else if (!strcmp(argv[i], "--pauli-rot") && i + 2 < argc) {
+            char *end;
+            rot[n_rot] = argv[++i];
+            rot_theta[n_rot] = strtod(argv[++i], &end);
+            if (end == argv[i] || *end) { printf("--pauli-rot \"%s\" %s: expected an angle\n", rot[n_rot], argv[i]); return 1; }
+            n_rot++;
+        }
         else if (!file) file = argv[i];
         else if (!have_m) { num_m = atol(argv[i]); have_m = 1; }
     }
@@ -135,6 +146,13 @@ int main(int argc, char **argv)
     rc = qsb_create(&s, nq, &o);
     if (!rc && load_state) rc = qsb_load_state(s, load_state);
     if (!rc) rc = qsb_apply_gates(s, gates, n);
+    if (!rc && n_rot) {   /* one call for all rotations: consecutive ones share sweeps over the state */
+        uint64_t *rx = (uint64_t *)malloc(sizeof(uint64_t) * 2 * n_rot);
+        if (!rx) { printf("Malloc error\n"); return 1; }
+        for (int k = 0; k < n_rot && !rc; k++) rc = qsb_pauli_from_string(rot[k], nq, &rx[k], &rx[n_rot + k]);
+        if (!rc) rc = qsb_apply_pauli_rotations(s, rx, rx + n_rot, rot_theta, (size_t)n_rot);
+        free(rx);
+    }
     if (!rc && save_state) rc = qsb_save_state(s, save_state);
     if (rc) { printf("%s\n", qsb_last_error()); return 1; }
     printf("%lf\n", now_s() - t0);
@@ -228,5 +246,7 @@ int main(int argc, char **argv)
     free(expect);
     free(marginal);
     free(rdm);
+    free(rot);
+    free(rot_theta);
     return 0;
 }

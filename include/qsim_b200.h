@@ -211,6 +211,31 @@ int qsb_pauli_from_string(const char *text, int num_qubits, uint64_t *x, uint64_
 int qsb_expectation_dry_run(int num_qubits, const qsb_options_t *opt, const uint64_t *x, const uint64_t *z,
                             size_t nterms, uint32_t *sweeps, uint32_t *exchanges);
 
+/* ---- Pauli rotations ---------------------------------------------------------
+ * Rotation k is R_k = exp(-i theta_k P_k / 2) = cos(theta_k / 2) I - i sin(theta_k / 2) P_k for the Pauli string P_k given
+ * as logical masks in the format of the observables above (x: X or Y, z: Z or Y), applied to the state as
+ *     a <- cos(theta_k / 2) a - i sin(theta_k / 2) (P_k a)      with (P_k a)_j from the action formula above,
+ * for k = 0, 1, ..., n - 1 in that order: the first listed rotation acts first, like a gate list.  x = z = 0 multiplies
+ * the state by exp(-i theta / 2) (kept, not dropped).  cos and sin are computed in fp64 on the host, the arithmetic is
+ * done in the state's precision, and nothing is renormalised.  theta = 0 is skipped: it leaves the state bytes as they
+ * are.  Note that "rz" in circuit text is the phase gate diag(1, e^{i theta}), while the rotation of "Z0" is
+ * diag(e^{-i theta / 2}, e^{i theta / 2}).
+ *
+ * Applied on the device in tile sweeps: a sweep carries a consecutive run of rotations whose X parts outside one tile of
+ * the state agree (diagonal rotations fit any run; n single-qubit X rotations on distinct qubits take about n / 9) and
+ * costs one read and one write of the local shard however many rotations it carries.  Rotations are never reordered.
+ * The qubit layout, the state buffer (a captured graph's state), the role of the exchange buffer and the peer mappings
+ * are left as they are, so a plan made before the call still executes after it.
+ * Errors return QSB_ERR_ARG with the state untouched: a null handle, a null array when n > 0, a qubit >= the handle's
+ * qubits, a non-finite theta.  n = 0 is a no-op.  A sharded handle without qsb_comm_init gives QSB_ERR_COMM.  On a
+ * sharded state the call is collective (same arguments on every rank): a sweep whose rotations flip rank qubits first
+ * receives the partner rank's shard into the exchange buffer, so it costs one shard copy, two reads and one write. */
+int qsb_apply_pauli_rotations(qsb_t *s, const uint64_t *x, const uint64_t *z, const double *theta, size_t n);
+/* Host only, no device: the number of sweeps (launches that read and write the shard) and partner-shard copies that
+ * qsb_apply_pauli_rotations would run for these rotations (all angles taken non-zero) from the identity layout. */
+int qsb_pauli_rotation_dry_run(int num_qubits, const qsb_options_t *opt, const uint64_t *x, const uint64_t *z,
+                               size_t n, uint32_t *sweeps, uint32_t *exchanges);
+
 /* ---- marginals and projective measurement ----------------------------------
  * The measured qubits are an array qubits[0..k-1] of distinct LOGICAL qubits, 1 <= k <= min(n, 20).  Bit i of a bin
  * index or an outcome is the value of qubits[i], so {3, 0} gives the transposed table of {0, 3}.  All sums are fp64
