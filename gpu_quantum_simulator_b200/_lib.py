@@ -69,6 +69,11 @@ SYMBOLS = {
     "qsb_apply_pauli_rotations": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
     "qsb_pauli_rotation_dry_run": (C.c_int, [C.c_int, C.POINTER(Options), C.c_void_p, C.c_void_p, C.c_size_t,
                                              C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+    "qsb_pauli_rotation_gradient": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p,
+                                              C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_double), C.c_void_p]),
+    "qsb_pauli_rotation_gradient_dry_run": (C.c_int, [C.c_int, C.POINTER(Options), C.c_void_p, C.c_void_p, C.c_size_t,
+                                                      C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_uint32),
+                                                      C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     "qsb_marginal_probabilities": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "qsb_collapse": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_uint64, C.POINTER(C.c_double)]),
     "qsb_measure_qubits": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.POINTER(C.c_uint64),

@@ -266,15 +266,6 @@ int pauli_dry_run_shape(int num_qubits, const qsb_options_t *opt_in, qsb_options
     return QSB_OK;
 }
 
-namespace {
-
-struct ExpSweep {
-    uint64_t xr = 0;               /* rank-bit flips: partner rank = rank ^ xr */
-    int8_t pb[16];                 /* tile coordinate bit j -> local physical bit */
-    uint64_t bmask = 0, x_out = 0; /* tile bits, local flips outside the tile */
-    std::vector<uint32_t> terms;
-};
-
 /* Greedy cover of the distinct physical x masks by sweeps (host only, no CUDA).  Sweeps come grouped by xr,
  * xr == 0 first, so that each partner shard is fetched once. */
 void exp_plan(int nloc, int T, int L, const std::vector<PhysTerm> &terms, std::vector<ExpSweep> &out)
@@ -327,17 +318,19 @@ void exp_plan(int nloc, int T, int L, const std::vector<PhysTerm> &terms, std::v
     }
 }
 
-uint32_t count_launches(const std::vector<ExpSweep> &sw)
-{
-    uint32_t n = 0;
-    for (auto &s : sw) n += (uint32_t)((s.terms.size() + EXP_KMAX - 1) / EXP_KMAX);
-    return n;
-}
-
 uint32_t count_exchanges(const std::vector<ExpSweep> &sw)
 {
     uint32_t n = 0; uint64_t last = 0;
     for (auto &s : sw) if (s.xr && s.xr != last) { n++; last = s.xr; }
+    return n;
+}
+
+namespace {
+
+uint32_t count_launches(const std::vector<ExpSweep> &sw)
+{
+    uint32_t n = 0;
+    for (auto &s : sw) n += (uint32_t)((s.terms.size() + EXP_KMAX - 1) / EXP_KMAX);
     return n;
 }
 

@@ -12,6 +12,9 @@
  *                       the reference keeps the state only in memory, quantum_simulator.c:75)
  *   --pauli-rot "X0 Z3" 0.25   (repeatable) the rotation exp(-i 0.25 P / 2) applied on the device after the circuit (after
  *                       --load-state, before --save-state), in flag order, so the lines below read the rotated state
+ *   --gradient "Z0 Z1" 0.5   (repeatable) a term 0.5 P of an observable H; with any, the --pauli-rot list is applied
+ *                       through the gradient call, which prints "ENERGY e" (<psi|H|psi>) and "GRADIENT g0 g1 ..." (dE/dtheta
+ *                       of each --pauli-rot angle in flag order, %.17g) after the --profile line
  *   --expect "Z0 Z1"    (repeatable) <psi|P|psi> of a Pauli string after the circuit, computed on the device:
  *                       one "EXPECTATION <text>: %.17g" line per flag, in flag order, after the --profile line
  *   --marginal "0 3 5"  (repeatable) marginal probabilities of these qubits after the circuit, computed on the device:
@@ -88,6 +91,9 @@ int main(int argc, char **argv)
     const char **rdm = (const char **)calloc((size_t)argc, sizeof(char *)); int n_rdm = 0;
     const char **rot = (const char **)calloc((size_t)argc, sizeof(char *)); int n_rot = 0;
     double *rot_theta = (double *)calloc((size_t)argc, sizeof(double));
+    const char **gterm = (const char **)calloc((size_t)argc, sizeof(char *)); int n_gterm = 0;
+    double *gcoef = (double *)calloc((size_t)argc, sizeof(double));
+    double energy = 0.0, *grad = (double *)calloc((size_t)argc, sizeof(double));
     for (int i = 1; i < argc; i++) {
         if (!strcmp(argv[i], "--precision") && i + 1 < argc) precision = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--dump-amplitudes")) dump = 1;
@@ -110,6 +116,13 @@ int main(int argc, char **argv)
             rot_theta[n_rot] = strtod(argv[++i], &end);
             if (end == argv[i] || *end) { printf("--pauli-rot \"%s\" %s: expected an angle\n", rot[n_rot], argv[i]); return 1; }
             n_rot++;
+        }
+        else if (!strcmp(argv[i], "--gradient") && i + 2 < argc) {
+            char *end;
+            gterm[n_gterm] = argv[++i];
+            gcoef[n_gterm] = strtod(argv[++i], &end);
+            if (end == argv[i] || *end) { printf("--gradient \"%s\" %s: expected a coefficient\n", gterm[n_gterm], argv[i]); return 1; }
+            n_gterm++;
         }
         else if (!file) file = argv[i];
         else if (!have_m) { num_m = atol(argv[i]); have_m = 1; }
@@ -146,11 +159,15 @@ int main(int argc, char **argv)
     rc = qsb_create(&s, nq, &o);
     if (!rc && load_state) rc = qsb_load_state(s, load_state);
     if (!rc) rc = qsb_apply_gates(s, gates, n);
-    if (!rc && n_rot) {   /* one call for all rotations: consecutive ones share sweeps over the state */
-        uint64_t *rx = (uint64_t *)malloc(sizeof(uint64_t) * 2 * n_rot);
+    if (!rc && (n_rot || n_gterm)) {   /* one call for all rotations: consecutive ones share sweeps over the state */
+        uint64_t *rx = (uint64_t *)malloc(sizeof(uint64_t) * 2 * (n_rot + n_gterm) + 16);
         if (!rx) { printf("Malloc error\n"); return 1; }
+        uint64_t *hx = rx + 2 * n_rot;
         for (int k = 0; k < n_rot && !rc; k++) rc = qsb_pauli_from_string(rot[k], nq, &rx[k], &rx[n_rot + k]);
-        if (!rc) rc = qsb_apply_pauli_rotations(s, rx, rx + n_rot, rot_theta, (size_t)n_rot);
+        for (int k = 0; k < n_gterm && !rc; k++) rc = qsb_pauli_from_string(gterm[k], nq, &hx[k], &hx[n_gterm + k]);
+        if (!rc && n_gterm)
+            rc = qsb_pauli_rotation_gradient(s, rx, rx + n_rot, rot_theta, (size_t)n_rot, hx, hx + n_gterm, gcoef, (size_t)n_gterm, &energy, grad);
+        else if (!rc) rc = qsb_apply_pauli_rotations(s, rx, rx + n_rot, rot_theta, (size_t)n_rot);
         free(rx);
     }
     if (!rc && save_state) rc = qsb_save_state(s, save_state);
@@ -164,6 +181,12 @@ int main(int argc, char **argv)
                nq, (unsigned long long)st.source_gates, st.passes, st.rounds, st.device_ms, st.plan_ms,
                (unsigned long long)st.bytes_moved, st.device_ms > 0 ? st.bytes_moved / st.device_ms * 1e-6 : 0.0,
                st.device_ms > 0 ? st.source_gates / st.device_ms * 1e3 : 0.0);
+    }
+    if (n_gterm) {
+        printf("ENERGY %.17g\n", energy);
+        printf("GRADIENT");
+        for (int k = 0; k < n_rot; k++) printf(" %.17g", grad[k]);
+        printf("\n");
     }
     if (n_expect) {   /* one call for all terms: they share the sweeps over the state */
         uint64_t *ex = (uint64_t *)malloc(sizeof(uint64_t) * 2 * n_expect);
@@ -248,5 +271,8 @@ int main(int argc, char **argv)
     free(rdm);
     free(rot);
     free(rot_theta);
+    free(gterm);
+    free(gcoef);
+    free(grad);
     return 0;
 }

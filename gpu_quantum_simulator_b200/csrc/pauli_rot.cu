@@ -41,42 +41,18 @@
 #include <vector>
 
 #include "pauli.h"
+#include "pauli_rot.cuh"
 #include "sim.h"
 #include "tiled.h"
 
 int tiled_comm_sendrecv(qsb_sim *s, const void *dsend, void *drecv, size_t bytes, int peer);
 int tiled_comm_allreduce_sum_u64(qsb_sim *s, void *dbuf, size_t count);
 
-#define ROT_THREADS 256
-#define ROT_TB 8                      /* thread bits of the tile coordinate */
 #define ROT_UNITS 2048                /* 16-byte units per tile: 2^12 f32 / 2^11 f64 amplitudes, 32 KiB */
 #define ROT_UB 11                     /* log2(ROT_UNITS) */
-#define ROT_KMAX 1024                 /* rotations per launch (one descriptor table) */
-#define ROT_TWO_PI 6.283185307179586
 
 /* a sweep reads pb[0..T-1], which exist because every shard has nloc >= tiled_min_local_bits() = QSB_T_* local bits */
 static_assert(12 <= QSB_T_F32 && 11 <= QSB_T_F64, "the rotation tile must fit the smallest shard");
-
-enum { ROT_DIAG = 1 };
-
-struct RotOp {                 /* one step of a launch: a pairing rotation or a stretch of diagonal rotations */
-    double c, s;               /* pairing: cos(t/2), +-sin(t/2) (the sign of Z on the own rank bits folded in) */
-    uint64_t zout;             /* pairing: Z on the local bits outside the tile, unit-address bits */
-    uint32_t xin, zin;         /* pairing: X / Z on the tile coordinate */
-    uint32_t flags;            /* ROT_DIAG; bits 1-2: slot flip; bits 3-4: Z parity of the slot bits; bits 5-6: w, the
-                                  factor -i * i^{popc(x&z)} = i^w */
-    uint32_t d0;               /* diagonal stretch: its terms, grouped by pattern, at d0 + poff[p] .. d0 + poff[p + 1] */
-    uint16_t poff[17];
-    uint16_t pad[3];
-};
-static_assert(sizeof(RotOp) == 80, "RotOp is 80 bytes");
-
-struct RotDiag {               /* one diagonal rotation of a stretch */
-    double theta;              /* the angle, negated if Z on the own rank bits has odd parity */
-    uint64_t zout;             /* Z on the local bits outside the tile, unit-address bits */
-    uint32_t zt;               /* Z on the thread bits of the tile coordinate */
-    uint32_t sp;               /* Z parity of the slot bits */
-};
 
 struct RotArgs {
     uint4 *A;                  /* own shard, read and written */
@@ -98,80 +74,6 @@ template <typename R> struct RotVec;
 template <> struct RotVec<float> { static constexpr int T = 12; };
 template <> struct RotVec<double> { static constexpr int T = 11; };
 
-/* (re, im) * i^w */
-template <typename R>
-__device__ __forceinline__ void mul_iw(R &re, R &im, uint32_t w)
-{
-    const R r = re, i = im;
-    switch (w) {
-    case 0: break;
-    case 1: re = -i; im = r; break;
-    case 2: re = -r; im = -i; break;
-    default: re = i; im = -r; break;
-    }
-}
-
-template <typename R>
-__device__ __forceinline__ void rot_pairs(R *sre, R *sim, const RotOp &op, uint64_t base, int ns, uint32_t tid)
-{
-    constexpr int T = RotVec<R>::T;
-    const uint32_t F = ((op.flags >> 1) & 3u) << T | op.xin;
-    const int h = 31 - __clz(F);
-    const uint32_t lowm = (1u << h) - 1, cmask = (1u << T) - 1, sp = (op.flags >> 3) & 3u, w = (op.flags >> 5) & 3u;
-    const uint32_t tpar = __popcll(base & op.zout) & 1;
-    const R c = (R)op.c, s = (R)op.s;
-    const uint32_t npairs = (uint32_t)ns << (T - 1);
-    for (uint32_t p = tid; p < npairs; p += ROT_THREADS) {
-        const uint32_t m0 = ((p & ~lowm) << 1) | (p & lowm), m1 = m0 ^ F;
-        const uint32_t par0 = (__popc(m0 & cmask & op.zin) + __popc((m0 >> T) & sp) + tpar) & 1;
-        const uint32_t par1 = (__popc(m1 & cmask & op.zin) + __popc((m1 >> T) & sp) + tpar) & 1;
-        const R a0r = sre[m0], a0i = sim[m0], a1r = sre[m1], a1i = sim[m1];
-        R t1r = a1r, t1i = a1i, t0r = a0r, t0i = a0i;
-        mul_iw(t1r, t1i, w);
-        mul_iw(t0r, t0i, w);
-        const R s1 = par1 ? -s : s, s0 = par0 ? -s : s;   /* new a_j = c a_j + s sigma_{j^x} i^w a_{j^x} */
-        sre[m0] = c * a0r + s1 * t1r; sim[m0] = c * a0i + s1 * t1i;
-        sre[m1] = c * a1r + s0 * t0r; sim[m1] = c * a1i + s0 * t0i;
-    }
-}
-
-template <typename R>
-__device__ __forceinline__ void rot_diag(R *sre, R *sim, const RotOp &op, const RotDiag *diag, uint64_t base, int ns, uint32_t tid)
-{
-    constexpr int T = RotVec<R>::T, NI = 1 << (T - ROT_TB);   /* amplitudes per thread and slot: m = tid | i << ROT_TB */
-    const RotDiag *d = diag + op.d0;
-    for (int slot = 0; slot < ns; slot++) {
-        double C[NI];
-#pragma unroll
-        for (int p = 0; p < NI; p++) {   /* C[p]: signed angle sum of the rotations whose Z on the bits of i is p */
-            double acc = 0.0;
-            for (int k = op.poff[p]; k < op.poff[p + 1]; k++) {
-                const RotDiag e = d[k];
-                const int par = (__popc(tid & e.zt) + __popcll(base & e.zout) + __popc((uint32_t)slot & e.sp)) & 1;
-                acc += par ? -e.theta : e.theta;
-            }
-            C[p] = acc;
-        }
-#pragma unroll
-        for (int hb = 1; hb < NI; hb <<= 1)   /* angle of amplitude i = sum_p C[p] (-1)^{popc(i & p)} */
-#pragma unroll
-            for (int i = 0; i < NI; i++)
-                if (!(i & hb)) { const double u = C[i], v = C[i + hb]; C[i] = u + v; C[i + hb] = u - v; }
-#pragma unroll
-        for (int i = 0; i < NI; i++) {
-            double ph = 0.5 * C[i];
-            ph -= ROT_TWO_PI * rint(ph * (1.0 / ROT_TWO_PI));
-            R cs, sn;
-            if (sizeof(R) == 4) { float fc, fs; sincosf((float)ph, &fs, &fc); cs = (R)fc; sn = (R)fs; }
-            else { double dc, ds; sincos(ph, &ds, &dc); cs = (R)dc; sn = (R)ds; }
-            const uint32_t m = ((uint32_t)slot << T) | ((uint32_t)i << ROT_TB) | tid;
-            const R re = sre[m], im = sim[m];   /* a * exp(-i ph) */
-            sre[m] = re * cs + im * sn;
-            sim[m] = im * cs - re * sn;
-        }
-    }
-}
-
 template <typename R>
 __global__ void __launch_bounds__(ROT_THREADS) k_pauli_rot(const __grid_constant__ RotArgs a)
 {
@@ -185,66 +87,23 @@ __global__ void __launch_bounds__(ROT_THREADS) k_pauli_rot(const __grid_constant
     for (uint64_t t = blockIdx.x; t < a.n_work; t += gridDim.x) {
         uint64_t base = 0;
         for (int i = 0; i < a.n_opos; i++) base |= ((t >> i) & 1ULL) << a.opos[i];
-        for (int slot = 0; slot < a.ns; slot++) {
-            const uint4 *src = (slot & a.so_rank) ? a.B : a.A;
-            const uint64_t ub = (base ^ ((slot & a.so_out) ? a.x_out : 0)) | toff;
-#pragma unroll
-            for (int k = 0; k < ROT_UNITS / ROT_THREADS; k++) {
-                uint64_t ko = 0;
-#pragma unroll
-                for (int b = 0; b < ROT_UB - ROT_TB; b++) if ((k >> b) & 1) ko |= a.uoff[ROT_TB + b];
-                const uint4 v = __ldcs(src + (ub | ko));
-                const uint32_t u = ((uint32_t)slot << ROT_UB) | tid | ((uint32_t)k << ROT_TB);
-                if (sizeof(R) == 4) {   /* unit { re0 re1 im0 im1 }: amplitudes 2u, 2u + 1 */
-                    reinterpret_cast<float2 *>(sre)[u] = make_float2(__uint_as_float(v.x), __uint_as_float(v.y));
-                    reinterpret_cast<float2 *>(sim)[u] = make_float2(__uint_as_float(v.z), __uint_as_float(v.w));
-                } else {                /* unit { re im } */
-                    reinterpret_cast<uint2 *>(sre)[u] = make_uint2(v.x, v.y);
-                    reinterpret_cast<uint2 *>(sim)[u] = make_uint2(v.z, v.w);
-                }
-            }
-        }
+        for (int slot = 0; slot < a.ns; slot++)
+            stage_tile<R, ROT_UB>(sre, sim, (slot & a.so_rank) ? a.B : a.A, (base ^ ((slot & a.so_out) ? a.x_out : 0)) | toff, a.uoff, slot, tid);
         __syncthreads();
         for (int j = 0; j < a.K; j++) {
             const RotOp &op = a.ops[j];
-            if (op.flags & ROT_DIAG) rot_diag<R>(sre, sim, op, a.diag, base, a.ns, tid);
-            else rot_pairs<R>(sre, sim, op, base, a.ns, tid);
+            if (op.flags & ROT_DIAG) rot_diag<R, T>(sre, sim, op, a.diag, base, a.ns, tid);
+            else rot_pairs<R, T>(sre, sim, op, base, a.ns, tid);
             __syncthreads();
         }
-        for (int slot = 0; slot < a.ns; slot++) {
-            if (slot & a.so_rank) continue;   /* the partner rank writes its own tiles */
-            const uint64_t ub = (base ^ ((slot & a.so_out) ? a.x_out : 0)) | toff;
-#pragma unroll
-            for (int k = 0; k < ROT_UNITS / ROT_THREADS; k++) {
-                uint64_t ko = 0;
-#pragma unroll
-                for (int b = 0; b < ROT_UB - ROT_TB; b++) if ((k >> b) & 1) ko |= a.uoff[ROT_TB + b];
-                const uint32_t u = ((uint32_t)slot << ROT_UB) | tid | ((uint32_t)k << ROT_TB);
-                uint4 v;
-                if (sizeof(R) == 4) {
-                    const float2 r = reinterpret_cast<const float2 *>(sre)[u], i = reinterpret_cast<const float2 *>(sim)[u];
-                    v = make_uint4(__float_as_uint(r.x), __float_as_uint(r.y), __float_as_uint(i.x), __float_as_uint(i.y));
-                } else {
-                    const uint2 r = reinterpret_cast<const uint2 *>(sre)[u], i = reinterpret_cast<const uint2 *>(sim)[u];
-                    v = make_uint4(r.x, r.y, i.x, i.y);
-                }
-                __stcs(a.A + (ub | ko), v);
-            }
-        }
+        for (int slot = 0; slot < a.ns; slot++)
+            if (!(slot & a.so_rank))   /* the partner rank writes its own tiles */
+                store_tile<R, ROT_UB>(a.A, sre, sim, (base ^ ((slot & a.so_out) ? a.x_out : 0)) | toff, a.uoff, slot, tid);
         __syncthreads();   /* the next tile group overwrites the planes */
     }
 }
 
 /* ================================================================================================ host */
-
-namespace {
-
-struct RotSweep {
-    uint64_t xr = 0;               /* rank-bit flips: partner rank = rank ^ xr */
-    int8_t pb[16];                 /* tile coordinate bit j -> local physical bit */
-    uint64_t bmask = 0, x_out = 0; /* tile bits, local flips outside the tile */
-    std::vector<uint32_t> rots;    /* indices into the rotation list, in list order */
-};
 
 /* Greedy grouping of the rotation list into sweeps, in order (host only, no CUDA). */
 void rot_plan(int nloc, int T, int L, const std::vector<PhysTerm> &rots, std::vector<RotSweep> &out)
@@ -290,7 +149,6 @@ uint32_t count_exchanges(const std::vector<RotSweep> &sw)
     return n;
 }
 
-/* slot bits of a sweep: the x_out partner tile and the partner rank's tiles */
 void slot_bits(const RotSweep &sw, int *so_out, int *so_rank, int *ns)
 {
     *so_out = sw.x_out ? 1 : 0;
@@ -298,11 +156,10 @@ void slot_bits(const RotSweep &sw, int *so_out, int *so_rank, int *ns)
     *ns = 1 << ((sw.x_out ? 1 : 0) + (sw.xr ? 1 : 0));
 }
 
-/* the launch table of one sweep: pairing rotations and diagonal stretches, in list order */
-void encode_sweep(const RotSweep &sw, const std::vector<PhysTerm> &pt, const std::vector<double> &theta, bool f32, int rank,
-                  std::vector<RotOp> &ops, std::vector<RotDiag> &diag)
+void encode_sweep(const RotSweep &sw, const std::vector<PhysTerm> &pt, const std::vector<double> &theta, int T, int su, int rank,
+                  std::vector<RotOp> &ops, std::vector<RotDiag> &diag, std::vector<uint32_t> *op_tags, std::vector<uint32_t> *diag_tags)
 {
-    const int T = f32 ? 12 : 11, su = f32 ? 1 : 0, NI = 1 << (T - ROT_TB);
+    const int NI = 1 << (T - ROT_TB);
     int so_out, so_rank, ns;
     slot_bits(sw, &so_out, &so_rank, &ns);
     size_t k = 0;
@@ -313,6 +170,7 @@ void encode_sweep(const RotSweep &sw, const std::vector<PhysTerm> &pt, const std
             op.flags = ROT_DIAG;
             op.d0 = (uint32_t)diag.size();
             std::vector<std::vector<RotDiag>> by(NI);
+            std::vector<std::vector<uint32_t>> tag_by(NI);
             for (; k < sw.rots.size() && !pt[sw.rots[k]].xl && !pt[sw.rots[k]].xr; k++) {
                 const PhysTerm &d = pt[sw.rots[k]];
                 const uint32_t zin = tile_coord(d.zl, sw.pb, T);
@@ -322,10 +180,12 @@ void encode_sweep(const RotSweep &sw, const std::vector<PhysTerm> &pt, const std
                 e.zt = zin & ((1u << ROT_TB) - 1);
                 e.sp = (uint32_t)(parity64(sw.x_out & d.zl) * so_out + parity64(sw.xr & d.zr) * so_rank);
                 by[zin >> ROT_TB].push_back(e);
+                tag_by[zin >> ROT_TB].push_back((uint32_t)k | (uint32_t)parity64((uint64_t)rank & d.zr) << 31);
             }
             for (int q = 0; q < NI; q++) {
                 op.poff[q + 1] = (uint16_t)(op.poff[q] + by[q].size());
                 diag.insert(diag.end(), by[q].begin(), by[q].end());
+                if (diag_tags) diag_tags->insert(diag_tags->end(), tag_by[q].begin(), tag_by[q].end());
             }
         } else {
             const double t = theta[sw.rots[k]];
@@ -337,11 +197,15 @@ void encode_sweep(const RotSweep &sw, const std::vector<PhysTerm> &pt, const std
             const uint32_t flip = ((p.xl & ~sw.bmask) ? so_out : 0) | (p.xr ? so_rank : 0);
             const uint32_t sp = (uint32_t)(parity64(sw.x_out & p.zl) * so_out + parity64(sw.xr & p.zr) * so_rank);
             op.flags = flip << 1 | sp << 3 | (uint32_t)((p.y + 3) & 3) << 5;
+            if (op_tags) op_tags->push_back((uint32_t)k | (uint32_t)parity64((uint64_t)rank & p.zr) << 31);
             k++;
         }
+        if (op_tags && (op.flags & ROT_DIAG)) op_tags->push_back(0);
         ops.push_back(op);
     }
 }
+
+namespace {
 
 struct DevMem {   /* scoped device allocation */
     void *p = nullptr;
@@ -402,7 +266,7 @@ extern "C" int qsb_apply_pauli_rotations(qsb_t *s, const uint64_t *x, const uint
     std::vector<RotOp> ops;
     std::vector<RotDiag> diag;
     std::vector<size_t> op0;
-    for (auto &w : sw) { op0.push_back(ops.size()); encode_sweep(w, pt, at, f32, s->rank, ops, diag); }
+    for (auto &w : sw) { op0.push_back(ops.size()); encode_sweep(w, pt, at, T, f32 ? 1 : 0, s->rank, ops, diag); }
     op0.push_back(ops.size());
     const size_t ops_bytes = ops.size() * sizeof(RotOp), diag_bytes = diag.size() * sizeof(RotDiag);
     DevMem mem;

@@ -131,6 +131,19 @@ def pauli_rotation_dry_run(num_qubits, paulis, precision=F32, world_size=1, low_
     return {"sweeps": sw.value, "exchanges": ex.value}
 
 
+def rotation_gradient_dry_run(num_qubits, paulis, observable, precision=F32, world_size=1, low_bits=0):
+    """Host-only: {"apply_sweeps", "adjoint_sweeps", "exchanges"} that Simulator.rotation_gradient would run besides
+    its forward pass and energy, from the identity qubit layout with every angle taken non-zero (apply_sweeps build
+    H psi, adjoint_sweeps walk the rotations backwards, exchanges = partner shards fetched by both)."""
+    x, z = pauli_masks(paulis, num_qubits)
+    hx, hz = pauli_masks(observable, num_qubits)
+    o = _options(precision, MODE_TILED, low_bits, 0, world_size, -1)
+    ap, ad, ex = C.c_uint32(), C.c_uint32(), C.c_uint32()
+    check(lib.qsb_pauli_rotation_gradient_dry_run(num_qubits, C.byref(o), x.ctypes.data, z.ctypes.data, x.size, hx.ctypes.data,
+                                                  hz.ctypes.data, hx.size, C.byref(ap), C.byref(ad), C.byref(ex)))
+    return {"apply_sweeps": ap.value, "adjoint_sweeps": ad.value, "exchanges": ex.value}
+
+
 class Plan:
     def __init__(self, sim, handle):
         self.sim, self.handle = sim, handle
@@ -329,6 +342,25 @@ class Simulator:
         else:
             step_p, step_t = texts + texts[::-1], np.concatenate([c * dt, (c * dt)[::-1]])
         self.apply_pauli_rotations(step_p * steps, np.tile(step_t, steps))
+
+    def rotation_gradient(self, paulis, thetas, observable, coeffs):
+        """Apply the rotations like apply_pauli_rotations and return (energy, grad): the energy
+        E = sum_j coeffs[j] <psi|observable[j]|psi> of the rotated state psi and the float64 array dE/dtheta_k, by the
+        adjoint method on the device.  The handle is left holding psi.  Sharded: collective, same arguments on every
+        rank, and every rank receives the same values."""
+        x, z = pauli_masks(paulis, self.num_qubits)
+        t = np.ascontiguousarray(np.asarray(thetas, dtype=np.float64).reshape(-1))
+        if t.size != x.size:
+            raise ValueError(f"{x.size} Pauli strings but {t.size} angles")
+        hx, hz = pauli_masks(observable, self.num_qubits)
+        c = np.ascontiguousarray(np.asarray(coeffs, dtype=np.float64).reshape(-1))
+        if c.size != hx.size:
+            raise ValueError(f"{hx.size} observable terms but {c.size} coefficients")
+        energy = C.c_double()
+        grad = np.empty(x.size, dtype=np.float64)
+        check(lib.qsb_pauli_rotation_gradient(self._h, x.ctypes.data, z.ctypes.data, t.ctypes.data, x.size, hx.ctypes.data,
+                                              hz.ctypes.data, c.ctypes.data, c.size, C.byref(energy), grad.ctypes.data))
+        return energy.value, grad
 
     # ---- marginals and projective measurement (bit i of a bin index or an outcome is the value of qubits[i])
     @staticmethod

@@ -236,6 +236,38 @@ int qsb_apply_pauli_rotations(qsb_t *s, const uint64_t *x, const uint64_t *z, co
 int qsb_pauli_rotation_dry_run(int num_qubits, const qsb_options_t *opt, const uint64_t *x, const uint64_t *z,
                                size_t n, uint32_t *sweeps, uint32_t *exchanges);
 
+/* ---- Pauli-rotation gradients -----------------------------------------------
+ * For the ansatz psi = R_{n-1} ... R_0 phi_0, R_k = exp(-i theta_k P_k / 2) (rotations rx / rz / theta in the format and
+ * order of qsb_apply_pauli_rotations, phi_0 the state in the handle at the call) and the observable H = sum_j coef[j] P_j
+ * (hx / hz in the format of the observables above, real coefficients):
+ *   - the handle is left holding psi, bit for bit what qsb_apply_pauli_rotations(s, rx, rz, theta, nrot) leaves (it is
+ *     that call); the qubit layout, the state buffer (a captured graph's state), the role of the exchange buffer and the
+ *     peer mappings are left as they are;
+ *   - *energy = sum_j coef[j] <psi|P_j|psi>, each value from qsb_expectation_pauli on psi, summed on the host in fp64 in
+ *     term order as e = e + coef[j] * v[j] from e = 0 (product rounded, then added), so it equals that sum by a caller;
+ *   - grad[k] = dE/dtheta_k = Im <lambda_k| P_k |phi_k>, phi_k = R_k ... R_0 phi_0, lambda_k = R_{k+1}^dag ... R_{n-1}^dag
+ *     H psi, by the adjoint method: one sweep set that builds H psi and one backward pass over the rotations.  It is for
+ *     the state as stored (nothing is renormalised); theta_k = 0 gets its gradient too.
+ * Reductions run in a fixed order without floating-point atomics: repeated calls return identical bits, and on a
+ * sharded state (a collective call, same arguments on every rank) every rank receives the same energy and gradients.
+ * nrot = 0 gives the energy only.  Device scratch, allocated before the state is touched and freed before the call
+ * returns: two shard-sized buffers on one GPU, three on a sharded state (at 30 qubits f32, 16 GiB beside the 8 GiB
+ * state), plus the launch tables and (CTAs x 1024) fp64 partials; QSB_ERR_NOMEM with the state untouched if it fails.
+ * Errors return QSB_ERR_ARG with the state untouched: a null handle, a null array when its count is > 0, nterms = 0, a
+ * null energy or (nrot > 0) grad, a qubit >= the handle's qubits, a non-finite theta or coefficient.  A sharded handle
+ * without qsb_comm_init gives QSB_ERR_COMM. */
+int qsb_pauli_rotation_gradient(qsb_t *s,
+                                const uint64_t *rx, const uint64_t *rz, const double *theta, size_t nrot,
+                                const uint64_t *hx, const uint64_t *hz, const double *coef, size_t nterms,
+                                double *energy, double *grad);
+/* Host only, no device, from the identity layout with every angle taken non-zero: the sweeps that build H psi, the
+ * fused adjoint sweeps, and the partner-shard copies of both.  The forward pass and the energy cost what
+ * qsb_pauli_rotation_dry_run and qsb_expectation_dry_run report. */
+int qsb_pauli_rotation_gradient_dry_run(int num_qubits, const qsb_options_t *opt,
+                                        const uint64_t *rx, const uint64_t *rz, size_t nrot,
+                                        const uint64_t *hx, const uint64_t *hz, size_t nterms,
+                                        uint32_t *apply_sweeps, uint32_t *adjoint_sweeps, uint32_t *exchanges);
+
 /* ---- marginals and projective measurement ----------------------------------
  * The measured qubits are an array qubits[0..k-1] of distinct LOGICAL qubits, 1 <= k <= min(n, 20).  Bit i of a bin
  * index or an outcome is the value of qubits[i], so {3, 0} gives the transposed table of {0, 3}.  All sums are fp64
