@@ -21,6 +21,11 @@ class Gate(C.Structure):
     _fields_ = [("controls", C.c_uint64), ("target", C.c_int32), ("flags", C.c_int32), ("m", C.c_double * 8)]
 
 
+class MatrixOp(C.Structure):
+    _fields_ = [("controls", C.c_uint64), ("k", C.c_int32), ("targets", C.c_int32 * 6), ("flags", C.c_int32),
+                ("m", C.POINTER(C.c_double))]
+
+
 class Options(C.Structure):
     _fields_ = [("precision", C.c_int32), ("device", C.c_int32), ("mode", C.c_int32), ("tile_bits", C.c_int32),
                 ("low_bits", C.c_int32), ("rank", C.c_int32), ("world_size", C.c_int32), ("use_graph", C.c_int32),
@@ -69,6 +74,9 @@ SYMBOLS = {
     "qsb_apply_pauli_rotations": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
     "qsb_pauli_rotation_dry_run": (C.c_int, [C.c_int, C.POINTER(Options), C.c_void_p, C.c_void_p, C.c_size_t,
                                              C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+    "qsb_apply_matrices": (C.c_int, [C.c_void_p, C.POINTER(MatrixOp), C.c_size_t]),
+    "qsb_matrix_dry_run": (C.c_int, [C.c_int, C.POINTER(Options), C.POINTER(MatrixOp), C.c_size_t, C.POINTER(C.c_uint32),
+                                     C.POINTER(C.c_uint32)]),
     "qsb_pauli_rotation_gradient": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p,
                                               C.c_void_p, C.c_void_p, C.c_size_t, C.POINTER(C.c_double), C.c_void_p]),
     "qsb_pauli_rotation_gradient_dry_run": (C.c_int, [C.c_int, C.POINTER(Options), C.c_void_p, C.c_void_p, C.c_size_t,

@@ -10,6 +10,11 @@
  *   <number_of_measurement> > 0 with --shots: "MEASUREMENT: <bits> (%ld)" (quantum_simulator.c:68-73)
  *   --save-state FILE / --load-state FILE   raw shard + qubit map after / before the circuit (checkpoint;
  *                       the reference keeps the state only in memory, quantum_simulator.c:75)
+ *   --matrix "0 3" FILE   (repeatable) the dense 2^k x 2^k matrix in FILE (2 * 4^k whitespace-separated numbers: re im,
+ *                       row-major; row / column index bit i = value of the i-th qubit listed) applied on the device after
+ *                       the circuit and --load-state; all --matrix flags go in flag order as one call, before --pauli-rot,
+ *                       --gradient and --save-state, so every later line reads the transformed state.  The files and
+ *                       qubit lists are checked before the circuit runs
  *   --pauli-rot "X0 Z3" 0.25   (repeatable) the rotation exp(-i 0.25 P / 2) applied on the device after the circuit (after
  *                       --load-state, before --save-state), in flag order, so the lines below read the rotated state
  *   --gradient "Z0 Z1" 0.5   (repeatable) a term 0.5 P of an observable H; with any, the --pauli-rot list is applied
@@ -94,6 +99,8 @@ int main(int argc, char **argv)
     const char **gterm = (const char **)calloc((size_t)argc, sizeof(char *)); int n_gterm = 0;
     double *gcoef = (double *)calloc((size_t)argc, sizeof(double));
     double energy = 0.0, *grad = (double *)calloc((size_t)argc, sizeof(double));
+    const char **mat_q = (const char **)calloc((size_t)argc, sizeof(char *)), **mat_f = (const char **)calloc((size_t)argc, sizeof(char *));
+    int n_mat = 0;
     for (int i = 1; i < argc; i++) {
         if (!strcmp(argv[i], "--precision") && i + 1 < argc) precision = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--dump-amplitudes")) dump = 1;
@@ -110,6 +117,7 @@ int main(int argc, char **argv)
         else if (!strcmp(argv[i], "--expect") && i + 1 < argc) expect[n_expect++] = argv[++i];
         else if (!strcmp(argv[i], "--marginal") && i + 1 < argc) marginal[n_marginal++] = argv[++i];
         else if (!strcmp(argv[i], "--rdm") && i + 1 < argc) rdm[n_rdm++] = argv[++i];
+        else if (!strcmp(argv[i], "--matrix") && i + 2 < argc) { mat_q[n_mat] = argv[++i]; mat_f[n_mat++] = argv[++i]; }
         else if (!strcmp(argv[i], "--pauli-rot") && i + 2 < argc) {
             char *end;
             rot[n_rot] = argv[++i];
@@ -129,6 +137,35 @@ int main(int argc, char **argv)
     }
     if (!file) { usage(argv[0]); return 1; }
     if (!have_seed) seed = (unsigned long long)time(NULL);   /* srand(time(NULL)), :46 */
+    /* --matrix files are read and checked before the circuit runs, so a bad file costs nothing */
+    qsb_matrix_op_t *mops = (qsb_matrix_op_t *)calloc((size_t)n_mat + 1, sizeof(qsb_matrix_op_t));
+    if (!mops) { printf("Malloc error\n"); return 1; }
+    for (int m = 0; m < n_mat; m++) {
+        int qs[64], k = 0;
+        if (!parse_qubits(mat_q[m], qs, &k) || k < 1 || k > QSB_MATRIX_MAX_K) {
+            printf("--matrix \"%s\": expected a whitespace-separated list of 1..%d qubits\n", mat_q[m], QSB_MATRIX_MAX_K); return 1;
+        }
+        const size_t want = (size_t)2 << (2 * k);
+        double *e = (double *)malloc(sizeof(double) * want);
+        FILE *f = fopen(mat_f[m], "r");
+        if (!e) { printf("Malloc error\n"); return 1; }
+        if (!f) { printf("--matrix \"%s\" %s: cannot open the file\n", mat_q[m], mat_f[m]); return 1; }
+        size_t got = 0;
+        double v;
+        while (got <= want && fscanf(f, "%lf", &v) == 1) { if (got < want) e[got] = v; got++; }
+        int ch;
+        while ((ch = fgetc(f)) == ' ' || ch == '\t' || ch == '\n' || ch == '\r') {}
+        const int clean = ch == EOF;   /* nothing but numbers and white space */
+        fclose(f);
+        if (got != want || !clean) {
+            printf("--matrix \"%s\" %s: expected %zu numbers (re im of a %d x %d matrix, row-major)%s\n", mat_q[m], mat_f[m],
+                   want, 1 << k, 1 << k, got > want ? ", found more" : !clean ? ", found text that is not a number" : "");
+            return 1;
+        }
+        mops[m].k = k;
+        for (int i = 0; i < k; i++) mops[m].targets[i] = qs[i];
+        mops[m].m = e;
+    }
 
     int nq = 0; qsb_gate_t *gates = NULL; size_t n = 0;
     int rc = qsb_parse_qasm_file(file, &nq, &gates, &n);
@@ -155,10 +192,13 @@ int main(int argc, char **argv)
         qsb_free(gates);
         return 0;
     }
+    /* the qubits and entries of every --matrix against the circuit's register, before the circuit runs */
+    if (n_mat && qsb_matrix_dry_run(nq, &o, mops, (size_t)n_mat, NULL, NULL)) { printf("%s\n", qsb_last_error()); return 1; }
     qsb_t *s = NULL;
     rc = qsb_create(&s, nq, &o);
     if (!rc && load_state) rc = qsb_load_state(s, load_state);
     if (!rc) rc = qsb_apply_gates(s, gates, n);
+    if (!rc && n_mat) rc = qsb_apply_matrices(s, mops, (size_t)n_mat);   /* one call: consecutive ops share sweeps */
     if (!rc && (n_rot || n_gterm)) {   /* one call for all rotations: consecutive ones share sweeps over the state */
         uint64_t *rx = (uint64_t *)malloc(sizeof(uint64_t) * 2 * (n_rot + n_gterm) + 16);
         if (!rx) { printf("Malloc error\n"); return 1; }
@@ -274,5 +314,9 @@ int main(int argc, char **argv)
     free(gterm);
     free(gcoef);
     free(grad);
+    for (int m = 0; m < n_mat; m++) free((void *)mops[m].m);
+    free(mops);
+    free(mat_q);
+    free(mat_f);
     return 0;
 }

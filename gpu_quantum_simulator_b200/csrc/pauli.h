@@ -1,5 +1,5 @@
-/* pauli.h -- Pauli-string helpers and sweep planners defined in expect.cu / pauli_rot.cu and shared with pauli_grad.cu
- * (host only, no CUDA calls). */
+/* pauli.h -- Pauli-string helpers and sweep planners defined in expect.cu / pauli_rot.cu / matrix.cu and shared with
+ * pauli_grad.cu (host only, no CUDA calls). */
 #pragma once
 #include <vector>
 #include "sim.h"
@@ -77,3 +77,25 @@ void slot_bits(const RotSweep &sw, int *so_out, int *so_rank, int *ns);
 void encode_sweep(const RotSweep &sw, const std::vector<PhysTerm> &pt, const std::vector<double> &theta, int T, int su, int rank,
                   std::vector<RotOp> &ops, std::vector<RotDiag> &diag, std::vector<uint32_t> *op_tags = nullptr,
                   std::vector<uint32_t> *diag_tags = nullptr);
+
+/* ---- dense-matrix grouping of matrix.cu */
+#define MAT_KMAX 1024                 /* matrix ops per launch (one descriptor table) */
+
+struct MatPhys {               /* one matrix op under the qubit layout, rank targets reduced to at most one */
+    uint64_t tl, tr;           /* targets on local physical bits / on rank bits (bit j = rank bit j) */
+    uint64_t cl, cr;           /* controls on local physical bits / on rank bits */
+    int k;
+    int8_t tq[8];              /* target i -> physical bit (>= nloc: rank bit tq - nloc) */
+};
+
+struct MatSweep {
+    uint64_t xr = 0;               /* rank-bit target of the run: partner rank = rank ^ xr */
+    int8_t pb[16];                 /* tile coordinate bit j -> local physical bit */
+    uint64_t bmask = 0;            /* tile bits */
+    std::vector<uint32_t> ops;     /* indices into the op list, in list order */
+};
+
+/* greedy grouping of the op list into sweeps of T tile bits, in order: a run ends at an op whose local targets do not
+ * fit the tile any more, at a second rank target that differs from the run's, or at MAT_KMAX ops.  false if an op fits
+ * no tile at all (more local targets outside the low bits than T - L) */
+bool matrix_plan(int nloc, int T, int L, const std::vector<MatPhys> &ops, std::vector<MatSweep> &out);

@@ -13,7 +13,7 @@ import os
 
 import numpy as np
 
-from ._lib import lib, check, Gate, Options, RunStats, F32, F64, MODE_TILED, MODE_SWEEP
+from ._lib import lib, check, Gate, MatrixOp, Options, RunStats, F32, F64, MODE_TILED, MODE_SWEEP
 
 
 def _gate_array(gates):
@@ -142,6 +142,51 @@ def rotation_gradient_dry_run(num_qubits, paulis, observable, precision=F32, wor
     check(lib.qsb_pauli_rotation_gradient_dry_run(num_qubits, C.byref(o), x.ctypes.data, z.ctypes.data, x.size, hx.ctypes.data,
                                                   hz.ctypes.data, hx.size, C.byref(ap), C.byref(ad), C.byref(ex)))
     return {"apply_sweeps": ap.value, "adjoint_sweeps": ad.value, "exchanges": ex.value}
+
+
+def _matrix_ops(ops, num_qubits=None):
+    """[(U, qubits) or (U, qubits, controls)] -> (ctypes array of MatrixOp, the numpy buffers its pointers address).
+    U is None in a dry run (only shapes are read); otherwise a (2^k, 2^k) complex array."""
+    arr = (MatrixOp * max(len(ops), 1))()
+    keep = []
+    for i, op in enumerate(ops):
+        U, qubits = op[0], [int(x) for x in np.atleast_1d(op[1])]
+        controls = [int(x) for x in np.atleast_1d(op[2])] if len(op) > 2 else []
+        if len(qubits) > 6:
+            raise ValueError(f"op {i}: {len(qubits)} targets, at most 6")
+        o = arr[i]
+        o.k = len(qubits)
+        for j, x in enumerate(qubits):
+            o.targets[j] = x
+        for c in controls:
+            if not 0 <= c < 64:
+                raise ValueError(f"op {i}: control {c} outside [0, 64)")
+            o.controls |= 1 << c
+        if U is not None:
+            d = 1 << len(qubits)
+            m = np.ascontiguousarray(np.asarray(U, dtype=np.complex128))
+            if m.shape != (d, d):
+                raise ValueError(f"op {i}: matrix of shape {m.shape} for {len(qubits)} targets, expected ({d}, {d})")
+            keep.append(m)
+            o.m = m.view(np.float64).ctypes.data_as(C.POINTER(C.c_double))
+    return arr, keep
+
+
+def matrix_dry_run(num_qubits, shapes, precision=F32, world_size=1, low_bits=0):
+    """Host-only: {"sweeps", "exchanges"} that Simulator.apply_matrices would run for ops of these shapes from the
+    identity qubit layout.  shapes: a list of target lists, or of (targets, controls) pairs (sweeps = reads and writes of
+    the local shard, exchanges = partner shards fetched, one per sweep with a target on a rank qubit)."""
+    ops = []
+    for sh in shapes:
+        if len(sh) == 2 and not np.isscalar(sh[0]):
+            ops.append((None, sh[0], sh[1]))
+        else:
+            ops.append((None, sh))
+    arr, _ = _matrix_ops(ops)
+    o = _options(precision, MODE_TILED, low_bits, 0, world_size, -1)
+    sw, ex = C.c_uint32(), C.c_uint32()
+    check(lib.qsb_matrix_dry_run(num_qubits, C.byref(o), arr, len(ops), C.byref(sw), C.byref(ex)))
+    return {"sweeps": sw.value, "exchanges": ex.value}
 
 
 class Plan:
@@ -361,6 +406,22 @@ class Simulator:
         check(lib.qsb_pauli_rotation_gradient(self._h, x.ctypes.data, z.ctypes.data, t.ctypes.data, x.size, hx.ctypes.data,
                                               hz.ctypes.data, c.ctypes.data, c.size, C.byref(energy), grad.ctypes.data))
         return energy.value, grad
+
+    # ---- dense matrices (bit i of a row or column index is the value of qubits[i])
+    def apply_matrix(self, U, qubits, controls=()):
+        """Apply the (2^k, 2^k) complex matrix U to the target qubits (k = len(qubits), 1..6): for every index whose
+        controls are all 1, a'[targets = r] = sum_c U[r, c] a[targets = c], so [3, 0] means the transposed qubit order of
+        [0, 3].  No unitarity check and no renormalisation; the arithmetic is in the state's precision.  The qubit
+        layout is left as it is.  Sharded: collective, same arguments on every rank."""
+        self.apply_matrices([(U, qubits, controls)])
+
+    def apply_matrices(self, ops):
+        """A list of (U, qubits) or (U, qubits, controls), applied in list order (the first acts first) as one call, so
+        consecutive ops share sweeps over the state."""
+        ops = list(ops)
+        arr, keep = _matrix_ops(ops)
+        check(lib.qsb_apply_matrices(self._h, arr, len(ops)))
+        del keep
 
     # ---- marginals and projective measurement (bit i of a bin index or an outcome is the value of qubits[i])
     @staticmethod

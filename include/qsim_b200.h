@@ -236,6 +236,49 @@ int qsb_apply_pauli_rotations(qsb_t *s, const uint64_t *x, const uint64_t *z, co
 int qsb_pauli_rotation_dry_run(int num_qubits, const qsb_options_t *opt, const uint64_t *x, const uint64_t *z,
                                size_t n, uint32_t *sweeps, uint32_t *exchanges);
 
+/* ---- dense matrices -----------------------------------------------------------
+ * A matrix op is a complex 2^k x 2^k matrix m on k distinct LOGICAL target qubits, 1 <= k <= QSB_MATRIX_MAX_K, optionally
+ * controlled.  For each op in list order (the first listed acts first, like a gate list) and every index j whose control
+ * bits are all 1:
+ *     a'[j with targets = r] = sum_c m[r][c] * a[j with targets = c]
+ * where bit i of a row / column index r, c is the value of targets[i] -- the index convention of the marginals and the
+ * reduced density matrices, so {3, 0} means the transposed qubit order of {0, 3}.  For k = 1 and the same entries this
+ * is exactly qsb_gate_t's  out0 = m00 a + m01 b.  Entries are fp64 on the host; the arithmetic is done in the state's
+ * precision, and each output is a sum in a fixed order (repeated calls return identical bits).  There is no unitarity
+ * check and nothing is renormalised: non-unitary matrices (Kraus operators, projectors, Hamiltonian blocks) are applied
+ * as they are.
+ *
+ * Applied on the device in tile sweeps: a sweep carries a consecutive run of ops whose targets fit one tile of the state
+ * and costs one read and one write of the local shard however many ops it carries.  Ops are never reordered.  The qubit
+ * layout, the state buffer (a captured graph's state), the role of the exchange buffer and the peer mappings are left as
+ * they are, so a plan made before the call still executes after it.
+ * Errors return QSB_ERR_ARG with the state untouched: a null handle, a null ops array when n > 0, k outside
+ * [1, min(n_qubits, QSB_MATRIX_MAX_K)], a target >= n_qubits or repeated, a control >= n_qubits or equal to a target, a
+ * null m, a non-finite entry, flags != 0, and options (the handle's, or a dry run's) whose low_bits is outside the range
+ * the tile scheduler accepts (f32 3..6, f64 2..5, 0 = the default), which leaves every tile room for any op.  n = 0 is a
+ * no-op.  A sharded handle without qsb_comm_init gives QSB_ERR_COMM.
+ * Device scratch is allocated once per call and freed before it returns: the launch table plus the matrices in the
+ * state's precision (at most 64 KiB per k = 6 op in f64); QSB_ERR_NOMEM leaves the state untouched.
+ * On a sharded state the call is collective (the same ops on every rank).  A sweep whose run has a target on a rank
+ * qubit first receives the partner rank's shard into the exchange buffer (one shard copy, two reads, one write).  An op
+ * with m >= 2 targets on rank qubits is applied as SWAP(r_i, l_i) ... U' ... SWAP(r_i, l_i) for i = 2..m, with l_i local
+ * qubits that are neither targets nor controls of the op standing in for r_i in U': 2 (m - 1) more sweeps and shard
+ * copies unless they merge with neighbours, and QSB_ERR_ARG if no such local qubit is free. */
+#define QSB_MATRIX_MAX_K 6
+typedef struct qsb_matrix_op {
+    uint64_t controls;                  /* bit q set: logical qubit q must be 1 for the matrix to act (as qsb_gate_t) */
+    int32_t k;                          /* number of targets, 1..QSB_MATRIX_MAX_K */
+    int32_t targets[QSB_MATRIX_MAX_K];  /* distinct logical qubits; bit i of a row / column index = value of targets[i] */
+    int32_t flags;                      /* reserved, 0 */
+    const double *m;                    /* 2 * 4^k doubles, row-major (re, im): entry (a, b) at m[2 * (a * 2^k + b)] */
+} qsb_matrix_op_t;
+
+int qsb_apply_matrices(qsb_t *s, const qsb_matrix_op_t *ops, size_t n);
+/* Host only, no device: the number of sweeps (launches that read and write the shard) and partner-shard copies that
+ * qsb_apply_matrices would run for these ops from the identity layout.  m may be NULL here: only shapes are read. */
+int qsb_matrix_dry_run(int num_qubits, const qsb_options_t *opt, const qsb_matrix_op_t *ops, size_t n,
+                       uint32_t *sweeps, uint32_t *exchanges);
+
 /* ---- Pauli-rotation gradients -----------------------------------------------
  * For the ansatz psi = R_{n-1} ... R_0 phi_0, R_k = exp(-i theta_k P_k / 2) (rotations rx / rz / theta in the format and
  * order of qsb_apply_pauli_rotations, phi_0 the state in the handle at the call) and the observable H = sum_j coef[j] P_j
