@@ -8,9 +8,9 @@ fallback -- importing works anywhere, running needs a CUDA device.
 from ._lib import lib, QsbError, Gate, MatrixOp, Options, RunStats, F32, F64, MODE_TILED, MODE_SWEEP, MODE_DENSE  # noqa: F401
 from .simulator import (Simulator, parse_qasm_file, parse_qasm_string, gates_from_circuit, plan_dry_run, sample_uniform,  # noqa: F401
                         expectation_dry_run, pauli_masks, pauli_rotation_dry_run, rotation_gradient_dry_run,
-                        matrix_dry_run)
+                        matrix_dry_run, overlap_dry_run)
 from . import circuits  # noqa: F401
 
 __all__ = ["Simulator", "parse_qasm_file", "parse_qasm_string", "gates_from_circuit", "plan_dry_run", "sample_uniform",
            "expectation_dry_run", "pauli_masks", "pauli_rotation_dry_run", "rotation_gradient_dry_run",
-           "matrix_dry_run", "circuits", "lib", "QsbError", "Gate", "MatrixOp", "Options", "RunStats", "F32", "F64", "MODE_TILED", "MODE_SWEEP", "MODE_DENSE"]
+           "matrix_dry_run", "overlap_dry_run", "circuits", "lib", "QsbError", "Gate", "MatrixOp", "Options", "RunStats", "F32", "F64", "MODE_TILED", "MODE_SWEEP", "MODE_DENSE"]

@@ -217,6 +217,16 @@ int exp_geometry(int prec, const qsb_options_t *opt, int *T, int *L)
     return QSB_OK;
 }
 
+int check_low_bits(int prec, const qsb_options_t *opt, const char *fn)
+{
+    const int lb = opt ? opt->low_bits : 0, lo = prec == QSB_F64 ? 2 : 3;
+    if (lb > 0 && (lb < lo || lb > lo + 3)) {
+        qsb_set_error("%s: low_bits %d unsupported for this precision (expected %d..%d, or 0 for the default)", fn, lb, lo, lo + 3);
+        return QSB_ERR_ARG;
+    }
+    return QSB_OK;
+}
+
 int check_terms(int n, const uint64_t *x, const uint64_t *z, size_t nterms, const char *fn)
 {
     if (nterms && (!x || !z)) { qsb_set_error("%s: null term array", fn); return QSB_ERR_ARG; }

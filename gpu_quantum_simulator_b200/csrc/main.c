@@ -28,6 +28,11 @@
  *   --rdm "0 3"         (repeatable) reduced density matrix of these qubits after the circuit, computed on the device:
  *                       one "RDM <qubits>: re_00 im_00 re_01 im_01 ..." line (%.17g, row-major, row / column index: bit i
  *                       = value of the i-th qubit listed) per flag, in flag order, after the MARGINAL lines
+ *   --overlap FILE      (repeatable) runs the circuit FILE from |0...0> on a second handle of the same precision and mode
+ *                       and prints "OVERLAP <file>: re im fidelity" (%.17g): <psi|phi> with psi the main state as it stands
+ *                       after --matrix, --pauli-rot and --gradient, phi FILE's state, fidelity |<psi|phi>|^2 / (<psi|psi>
+ *                       <phi|phi>), computed on the device; one line per flag, in flag order, after the RDM lines.  FILE
+ *                       is parsed and its qubit count checked before the main circuit runs
  *   --plan-only [--gpus N]   host-side fusion only (no GPU needed): one JSON line with the passes, rounds, ops and
  *                       qubit exchanges the circuit would run as on N ranks, instead of running it
  * Errors go to stdout followed by exit(1), like the reference (:56,:129,:213-219).
@@ -101,6 +106,7 @@ int main(int argc, char **argv)
     double energy = 0.0, *grad = (double *)calloc((size_t)argc, sizeof(double));
     const char **mat_q = (const char **)calloc((size_t)argc, sizeof(char *)), **mat_f = (const char **)calloc((size_t)argc, sizeof(char *));
     int n_mat = 0;
+    const char **ovl = (const char **)calloc((size_t)argc, sizeof(char *)); int n_ovl = 0;
     for (int i = 1; i < argc; i++) {
         if (!strcmp(argv[i], "--precision") && i + 1 < argc) precision = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--dump-amplitudes")) dump = 1;
@@ -117,6 +123,7 @@ int main(int argc, char **argv)
         else if (!strcmp(argv[i], "--expect") && i + 1 < argc) expect[n_expect++] = argv[++i];
         else if (!strcmp(argv[i], "--marginal") && i + 1 < argc) marginal[n_marginal++] = argv[++i];
         else if (!strcmp(argv[i], "--rdm") && i + 1 < argc) rdm[n_rdm++] = argv[++i];
+        else if (!strcmp(argv[i], "--overlap") && i + 1 < argc) ovl[n_ovl++] = argv[++i];
         else if (!strcmp(argv[i], "--matrix") && i + 2 < argc) { mat_q[n_mat] = argv[++i]; mat_f[n_mat++] = argv[++i]; }
         else if (!strcmp(argv[i], "--pauli-rot") && i + 2 < argc) {
             char *end;
@@ -191,6 +198,15 @@ int main(int argc, char **argv)
                st.swaps, (unsigned long long)st.bytes_moved, (unsigned long long)st.bytes_exchanged, st.plan_ms, qsb_version());
         qsb_free(gates);
         return 0;
+    }
+    /* every --overlap circuit is parsed and its register checked before the main circuit runs */
+    qsb_gate_t **ovl_g = (qsb_gate_t **)calloc((size_t)n_ovl + 1, sizeof(qsb_gate_t *));
+    size_t *ovl_n = (size_t *)calloc((size_t)n_ovl + 1, sizeof(size_t));
+    if (!ovl_g || !ovl_n) { printf("Malloc error\n"); return 1; }
+    for (int m = 0; m < n_ovl; m++) {
+        int oq = 0;
+        if (qsb_parse_qasm_file(ovl[m], &oq, &ovl_g[m], &ovl_n[m])) { printf("--overlap %s: %s\n", ovl[m], qsb_last_error()); return 1; }
+        if (oq != nq) { printf("--overlap %s: the circuit has %d qubits, the main circuit %d\n", ovl[m], oq, nq); return 1; }
     }
     /* the qubits and entries of every --matrix against the circuit's register, before the circuit runs */
     if (n_mat && qsb_matrix_dry_run(nq, &o, mops, (size_t)n_mat, NULL, NULL)) { printf("%s\n", qsb_last_error()); return 1; }
@@ -269,6 +285,18 @@ int main(int argc, char **argv)
         printf("\n");
         free(rho);
     }
+    for (int m = 0; m < n_ovl; m++) {
+        qsb_t *s2 = NULL;
+        double ov[2], nr[2];
+        rc = qsb_create(&s2, nq, &o);
+        if (!rc) rc = qsb_apply_gates(s2, ovl_g[m], ovl_n[m]);
+        if (!rc) rc = qsb_inner_product(s, s2, ov, nr);
+        if (rc) { printf("%s\n", qsb_last_error()); return 1; }
+        const double den = nr[0] * nr[1];
+        printf("OVERLAP %s: %.17g %.17g %.17g\n", ovl[m], ov[0], ov[1], (ov[0] * ov[0] + ov[1] * ov[1]) / den);   /* nan for a zero state */
+        qsb_destroy(s2);
+        qsb_free(ovl_g[m]);
+    }
     const unsigned long long N = 1ULL << nq;
     if (dump || dump_bin) {
         const unsigned long long chunk = 1ULL << 20;
@@ -309,6 +337,9 @@ int main(int argc, char **argv)
     free(expect);
     free(marginal);
     free(rdm);
+    free(ovl);
+    free(ovl_g);
+    free(ovl_n);
     free(rot);
     free(rot_theta);
     free(gterm);

@@ -314,11 +314,8 @@ void to_phys(int nloc, const BitPerm &perm, const std::vector<MatLog> &lg, std::
  * 3..6, f64 2..5, 0 = the default): in that range T - L >= QSB_MATRIX_MAX_K, so every op fits one tile. */
 int matrix_geometry(int prec, const qsb_options_t *opt, int *T, int *L, const char *fn)
 {
-    const int lb = opt ? opt->low_bits : 0, lo = prec == QSB_F64 ? 2 : 3;
-    if (lb > 0 && (lb < lo || lb > lo + 3)) {
-        qsb_set_error("%s: low_bits %d unsupported for this precision (expected %d..%d, or 0 for the default)", fn, lb, lo, lo + 3);
-        return QSB_ERR_ARG;
-    }
+    const int rc = check_low_bits(prec, opt, fn);
+    if (rc) return rc;
     exp_geometry(prec, opt, T, L);
     if (*T - *L < QSB_MATRIX_MAX_K) { qsb_set_error("%s: internal: %d free tile bits", fn, *T - *L); return QSB_ERR_ARG; }
     return QSB_OK;

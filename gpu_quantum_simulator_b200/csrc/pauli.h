@@ -10,6 +10,9 @@ inline int parity64(uint64_t v) { return __builtin_popcountll(v) & 1; }
 
 /* tile bits T (12 f32 / 11 f64) and the low bits L every tile keeps, for a precision and the handle's options */
 int exp_geometry(int prec, const qsb_options_t *opt, int *T, int *L);
+/* QSB_ERR_ARG (with a message naming fn) for a low_bits outside the range the tile scheduler accepts (f32 3..6, f64 2..5,
+ * 0 = the default) */
+int check_low_bits(int prec, const qsb_options_t *opt, const char *fn);
 /* QSB_ERR_ARG (with a message naming fn) for a null array when nterms > 0 or a qubit >= n */
 int check_terms(int n, const uint64_t *x, const uint64_t *z, size_t nterms, const char *fn);
 /* logical masks -> physical local / rank-bit masks under the layout perm */

@@ -180,15 +180,21 @@ int tiled_comm_allreduce_sum_u64(qsb_sim *s, void *dbuf, size_t count)
     return QSB_OK;
 }
 
-/* one send / receive pair with `peer` (expectation values: the partner shard of terms that flip rank bits) */
-int tiled_comm_sendrecv(qsb_sim *s, const void *dsend, void *drecv, size_t bytes, int peer)
+/* one grouped send to send_peer and receive from recv_peer (overlaps: the B shard goes to one rank and comes from another) */
+int tiled_comm_sendrecv_peers(qsb_sim *s, const void *dsend, int send_peer, void *drecv, int recv_peer, size_t bytes)
 {
     if (!s->comm) { qsb_set_error("sharded readout needs qsb_comm_init first"); return QSB_ERR_COMM; }
     QSB_NCCL(g_nccl.GroupStart());
-    QSB_NCCL(g_nccl.Send(dsend, bytes, 1 /* ncclUint8 */, peer, (qsb_nccl_comm_t)s->comm, s->stream));
-    QSB_NCCL(g_nccl.Recv(drecv, bytes, 1, peer, (qsb_nccl_comm_t)s->comm, s->stream));
+    QSB_NCCL(g_nccl.Send(dsend, bytes, 1 /* ncclUint8 */, send_peer, (qsb_nccl_comm_t)s->comm, s->stream));
+    QSB_NCCL(g_nccl.Recv(drecv, bytes, 1, recv_peer, (qsb_nccl_comm_t)s->comm, s->stream));
     QSB_NCCL(g_nccl.GroupEnd());
     return QSB_OK;
+}
+
+/* one send / receive pair with `peer` (expectation values: the partner shard of terms that flip rank bits) */
+int tiled_comm_sendrecv(qsb_sim *s, const void *dsend, void *drecv, size_t bytes, int peer)
+{
+    return tiled_comm_sendrecv_peers(s, dsend, peer, drecv, peer, bytes);
 }
 
 void tiled_comm_destroy(qsb_sim *s)

@@ -189,6 +189,23 @@ def matrix_dry_run(num_qubits, shapes, precision=F32, world_size=1, low_bits=0):
     return {"sweeps": sw.value, "exchanges": ex.value}
 
 
+def overlap_dry_run(num_qubits, perm_a, perm_b, precision_a=F32, precision_b=F32, world_size=1, rank=0, low_bits_a=0,
+                    low_bits_b=0):
+    """Host-only: {"steps", "exchanges"} that Simulator.overlap would run on `rank` for handles with these qubit layouts
+    (perm[q] = physical bit of qubit q, the format of Simulator.layout; bits >= the local bits are rank bits): steps =
+    partner shards of the other state combined, exchanges = those that are copied from another rank."""
+    pa = np.zeros(64, dtype=np.int8)
+    pb = np.zeros(64, dtype=np.int8)
+    pa[:num_qubits] = np.asarray(perm_a, dtype=np.int64)[:num_qubits]
+    pb[:num_qubits] = np.asarray(perm_b, dtype=np.int64)[:num_qubits]
+    oa = _options(precision_a, MODE_TILED, low_bits_a, rank, world_size, -1)
+    ob = _options(precision_b, MODE_TILED, low_bits_b, rank, world_size, -1)
+    st, ex = C.c_uint32(), C.c_uint32()
+    check(lib.qsb_inner_product_dry_run(num_qubits, C.byref(oa), pa.ctypes.data, C.byref(ob), pb.ctypes.data, C.byref(st),
+                                        C.byref(ex)))
+    return {"steps": st.value, "exchanges": ex.value}
+
+
 class Plan:
     def __init__(self, sim, handle):
         self.sim, self.handle = sim, handle
@@ -484,6 +501,31 @@ class Simulator:
         w = np.linalg.eigvalsh(rho / tr)
         w = w[w > 0.0]
         return float(-np.sum(w * np.log(w)) / np.log(base))
+
+    # ---- overlaps and state copy
+    def _inner(self, other):
+        out = np.empty(2, dtype=np.float64)
+        norms = np.empty(2, dtype=np.float64)
+        check(lib.qsb_inner_product(self._h, other._h, out.ctypes.data, norms.ctypes.data))
+        return complex(out[0], out[1]), float(norms[0]), float(norms[1])
+
+    def overlap(self, other):
+        """<self|other> = sum_j conj(self_j) other_j as a complex, in fp64 on the device over the states as stored (nothing
+        is renormalised).  The precisions and qubit layouts may differ; the states and layouts are left as they are.
+        Sharded: collective, every rank receives the same bits."""
+        return self._inner(other)[0]
+
+    def fidelity(self, other):
+        """|<self|other>|^2 / (<self|self> <other|other>) from one device call; ValueError if either norm is 0."""
+        ov, na, nb = self._inner(other)
+        if na == 0.0 or nb == 0.0:
+            raise ValueError(f"a state has norm 0 (norms {na}, {nb}): no fidelity")
+        return (ov.real * ov.real + ov.imag * ov.imag) / (na * nb)
+
+    def copy_from(self, other):
+        """This handle's amplitudes and qubit layout become other's (a device-to-device copy of the shard; same qubits,
+        precision, world, rank and device).  Plans made for the old layout are then refused, as after any layout change."""
+        check(lib.qsb_copy_state(self._h, other._h))
 
     def save_state(self, path):
         """Dump this rank's shard (device dtype, physical order) with its qubit map; one file per rank."""

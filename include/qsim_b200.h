@@ -363,6 +363,41 @@ int qsb_reset_qubits(qsb_t *s, const int *qubits, int k, double r, uint64_t *out
  * measured rank qubits (2^m - 1 shard copies per call), and every rank receives the same bits. */
 int qsb_reduced_density_matrix(qsb_t *s, const int *qubits, int k, double *rho);
 
+/* ---- overlaps and state copy ------------------------------------------------
+ * Two handles a, b of the same number of qubits, world size and rank, on the same device; otherwise QSB_ERR_ARG with
+ * the states untouched.  Precisions may differ (f32 with f32, f32 with f64 in either order, f64 with f64), the qubit
+ * layouts may differ arbitrarily, and a == b (the same handle twice) is allowed.
+ *
+ * qsb_inner_product computes, in fp64 on the states as stored (nothing is renormalised):
+ *     out[0] + i out[1] = <a|b> = sum_j conj(a_j) b_j        over the 2^n LOGICAL amplitudes,
+ * and, when norms is not NULL, norms[0] = <a|a> and norms[1] = <b|b> from the same read.  Every amplitude is converted to
+ * fp64 first; Re adds ar*br + ai*bi, the norms add the same expression, and Im adds ar*bi - ai*br, each product rounded on
+ * its own.  So for a == b, and for b just filled by qsb_copy_state(b, a), out[1] is exactly 0 and out[0] == norms[0] ==
+ * norms[1] bit for bit.  Reductions run in a fixed order without floating-point atomics: repeated calls return identical
+ * bits.  Neither state, qubit layout, state buffer (a captured graph's state), role of the exchange buffer nor peer
+ * mapping changes, so a plan made on either handle before the call still executes after it.
+ * Errors: a null handle or out, handles that differ as above, and options of either handle whose low_bits is outside the
+ * range the tile scheduler accepts (f32 3..6, f64 2..5, 0 = the default) give QSB_ERR_ARG; a sharded handle without
+ * qsb_comm_init on either side gives QSB_ERR_COMM.  Device scratch (per-CTA partials) is one allocation per call, freed
+ * before it returns; QSB_ERR_NOMEM leaves the states untouched.
+ * Cost: one read of a's shard in total.  On a sharded state the call is collective (same arguments on every rank) and
+ * every rank receives the same bits.  With R_a, R_b the qubits on the rank bits and d = |R_a \ R_b|, it runs 2^d steps;
+ * a step combines this rank's slice of a with the b shard of one partner rank, received into b's exchange buffer when it
+ * is not the own one: 2^d - 1 or 2^d shard copies when the rank qubits differ (2^g - 1 when the sets are disjoint), none
+ * when they sit on the same rank bits.  A call that copied a shard ends with an all-reduce on b's communicator. */
+int qsb_inner_product(qsb_t *a, qsb_t *b, double out[2], double norms[2]);
+/* dst's amplitudes and qubit layout become src's: on each rank a device-to-device copy of the shard as it lies plus the
+ * layout (no communication, but on a sharded state every rank calls it).  dst keeps its own state buffer.  The handles
+ * must have the same qubits, world, rank, device AND precision (else QSB_ERR_ARG); dst == src is a no-op.  Plans made
+ * on dst for its old layout are then refused by qsb_execute, as for any layout change. */
+int qsb_copy_state(qsb_t *dst, const qsb_t *src);
+/* Host only: the steps (partner b shards combined, one launch each) and the partner-shard copies that qsb_inner_product
+ * would run on rank opt_a->rank for handles with these options and layouts (perm64 format of qsb_get_layout: perm[q] =
+ * physical bit of qubit q, for q < num_qubits).  QSB_ERR_ARG for a layout that is not a permutation of the physical bits,
+ * options that differ in world size or rank, or a low_bits outside the accepted range. */
+int qsb_inner_product_dry_run(int num_qubits, const qsb_options_t *opt_a, const int8_t *perm_a,
+                              const qsb_options_t *opt_b, const int8_t *perm_b, uint32_t *steps, uint32_t *exchanges);
+
 /* ---- shard dump / reload ----------------------------------------------------
  * The reference keeps the state only in memory (quantum_simulator.c:75 frees it
  * at exit); long sharded runs want a checkpoint.  File = 128-byte header (magic
