@@ -26,6 +26,11 @@ class MatrixOp(C.Structure):
                 ("m", C.POINTER(C.c_double))]
 
 
+class Channel(C.Structure):
+    _fields_ = [("k", C.c_int32), ("targets", C.c_int32 * 4), ("nkraus", C.c_int32), ("flags", C.c_int32),
+                ("kraus", C.POINTER(C.c_double))]
+
+
 class Options(C.Structure):
     _fields_ = [("precision", C.c_int32), ("device", C.c_int32), ("mode", C.c_int32), ("tile_bits", C.c_int32),
                 ("low_bits", C.c_int32), ("rank", C.c_int32), ("world_size", C.c_int32), ("use_graph", C.c_int32),
@@ -92,6 +97,9 @@ SYMBOLS = {
     "qsb_copy_state": (C.c_int, [C.c_void_p, C.c_void_p]),
     "qsb_inner_product_dry_run": (C.c_int, [C.c_int, C.POINTER(Options), C.c_void_p, C.POINTER(Options), C.c_void_p,
                                             C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+    "qsb_apply_channels": (C.c_int, [C.c_void_p, C.POINTER(Channel), C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "qsb_channel_dry_run": (C.c_int, [C.c_int, C.POINTER(Options), C.POINTER(Channel), C.c_size_t, C.POINTER(C.c_uint32),
+                                      C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     "qsb_save_state": (C.c_int, [C.c_void_p, C.c_char_p]),
     "qsb_load_state": (C.c_int, [C.c_void_p, C.c_char_p]),
     "qsb_comm_unique_id": (C.c_int, [C.c_void_p]),

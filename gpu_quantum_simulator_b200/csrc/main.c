@@ -15,6 +15,14 @@
  *                       the circuit and --load-state; all --matrix flags go in flag order as one call, before --pauli-rot,
  *                       --gradient and --save-state, so every later line reads the transformed state.  The files and
  *                       qubit lists are checked before the circuit runs
+ *   --channel "0 3" FILE   (repeatable) a noise channel: FILE holds its Kraus operators, one after another, as
+ *                       whitespace-separated numbers (re im, row-major, 2 * 4^k per operator; row / column index bit i = value
+ *                       of the i-th qubit listed).  All --channel flags go in flag order as one quantum-trajectory call right
+ *                       after --matrix and before --pauli-rot, --gradient and --save-state; the branch of the c-th flag is
+ *                       drawn with r = qsb_sample_uniform(S, c), S from --channel-seed S (default 0; --seed drives the shots
+ *                       only).  One "CHANNEL <qubits>: <branch> <prob %.17g>" line per flag, in flag order, after the
+ *                       --profile line.  The files and qubit lists are checked with qsb_channel_dry_run before the circuit
+ *                       runs
  *   --pauli-rot "X0 Z3" 0.25   (repeatable) the rotation exp(-i 0.25 P / 2) applied on the device after the circuit (after
  *                       --load-state, before --save-state), in flag order, so the lines below read the rotated state
  *   --gradient "Z0 Z1" 0.5   (repeatable) a term 0.5 P of an observable H; with any, the --pauli-rot list is applied
@@ -106,6 +114,9 @@ int main(int argc, char **argv)
     double energy = 0.0, *grad = (double *)calloc((size_t)argc, sizeof(double));
     const char **mat_q = (const char **)calloc((size_t)argc, sizeof(char *)), **mat_f = (const char **)calloc((size_t)argc, sizeof(char *));
     int n_mat = 0;
+    const char **ch_q = (const char **)calloc((size_t)argc, sizeof(char *)), **ch_f = (const char **)calloc((size_t)argc, sizeof(char *));
+    int n_ch = 0;
+    unsigned long long ch_seed = 0;
     const char **ovl = (const char **)calloc((size_t)argc, sizeof(char *)); int n_ovl = 0;
     for (int i = 1; i < argc; i++) {
         if (!strcmp(argv[i], "--precision") && i + 1 < argc) precision = atoi(argv[++i]);
@@ -125,6 +136,8 @@ int main(int argc, char **argv)
         else if (!strcmp(argv[i], "--rdm") && i + 1 < argc) rdm[n_rdm++] = argv[++i];
         else if (!strcmp(argv[i], "--overlap") && i + 1 < argc) ovl[n_ovl++] = argv[++i];
         else if (!strcmp(argv[i], "--matrix") && i + 2 < argc) { mat_q[n_mat] = argv[++i]; mat_f[n_mat++] = argv[++i]; }
+        else if (!strcmp(argv[i], "--channel") && i + 2 < argc) { ch_q[n_ch] = argv[++i]; ch_f[n_ch++] = argv[++i]; }
+        else if (!strcmp(argv[i], "--channel-seed") && i + 1 < argc) ch_seed = strtoull(argv[++i], NULL, 10);
         else if (!strcmp(argv[i], "--pauli-rot") && i + 2 < argc) {
             char *end;
             rot[n_rot] = argv[++i];
@@ -173,6 +186,42 @@ int main(int argc, char **argv)
         for (int i = 0; i < k; i++) mops[m].targets[i] = qs[i];
         mops[m].m = e;
     }
+    /* --channel files are read before the circuit runs too; their qubits are checked below with the dry run */
+    qsb_channel_t *chs = (qsb_channel_t *)calloc((size_t)n_ch + 1, sizeof(qsb_channel_t));
+    double *ch_r = (double *)calloc((size_t)n_ch + 1, sizeof(double)), *ch_p = (double *)calloc((size_t)n_ch + 1, sizeof(double));
+    uint32_t *ch_b = (uint32_t *)calloc((size_t)n_ch + 1, sizeof(uint32_t));
+    if (!chs || !ch_r || !ch_p || !ch_b) { printf("Malloc error\n"); return 1; }
+    for (int m = 0; m < n_ch; m++) {
+        int qs[64], k = 0;
+        if (!parse_qubits(ch_q[m], qs, &k) || k < 1 || k > QSB_CHANNEL_MAX_K) {
+            printf("--channel \"%s\": expected a whitespace-separated list of 1..%d qubits\n", ch_q[m], QSB_CHANNEL_MAX_K); return 1;
+        }
+        const size_t per = (size_t)2 << (2 * k), cap = per << (2 * k);   /* at most 4^k operators */
+        double *e = (double *)malloc(sizeof(double) * cap);
+        FILE *f = fopen(ch_f[m], "r");
+        if (!e) { printf("Malloc error\n"); return 1; }
+        if (!f) { printf("--channel \"%s\" %s: cannot open the file\n", ch_q[m], ch_f[m]); return 1; }
+        size_t got = 0;
+        double v;
+        while (got <= cap && fscanf(f, "%lf", &v) == 1) { if (got < cap) e[got] = v; got++; }
+        int c;
+        while ((c = fgetc(f)) == ' ' || c == '\t' || c == '\n' || c == '\r') {}
+        const int clean = c == EOF;   /* nothing but numbers and white space */
+        fclose(f);
+        if (!got || got % per || got > cap || !clean) {
+            printf("--channel \"%s\" %s: expected 1..%d operators of %zu numbers each (re im of a %d x %d matrix, row-major), ",
+                   ch_q[m], ch_f[m], 1 << (2 * k), per, 1 << k, 1 << k);
+            if (got > cap) printf("found more than %d operators\n", 1 << (2 * k));   /* reading stopped at cap + 1 numbers */
+            else if (!clean) printf("found text that is not a number after %zu numbers\n", got);
+            else printf("found %zu numbers\n", got);
+            return 1;
+        }
+        chs[m].k = k;
+        for (int i = 0; i < k; i++) chs[m].targets[i] = qs[i];
+        chs[m].nkraus = (int32_t)(got / per);
+        chs[m].kraus = e;
+        ch_r[m] = qsb_sample_uniform(ch_seed, m);
+    }
 
     int nq = 0; qsb_gate_t *gates = NULL; size_t n = 0;
     int rc = qsb_parse_qasm_file(file, &nq, &gates, &n);
@@ -210,11 +259,14 @@ int main(int argc, char **argv)
     }
     /* the qubits and entries of every --matrix against the circuit's register, before the circuit runs */
     if (n_mat && qsb_matrix_dry_run(nq, &o, mops, (size_t)n_mat, NULL, NULL)) { printf("%s\n", qsb_last_error()); return 1; }
+    /* the qubits, operators and tile fit of every --channel against the circuit's register */
+    if (n_ch && qsb_channel_dry_run(nq, &o, chs, (size_t)n_ch, NULL, NULL, NULL)) { printf("%s\n", qsb_last_error()); return 1; }
     qsb_t *s = NULL;
     rc = qsb_create(&s, nq, &o);
     if (!rc && load_state) rc = qsb_load_state(s, load_state);
     if (!rc) rc = qsb_apply_gates(s, gates, n);
     if (!rc && n_mat) rc = qsb_apply_matrices(s, mops, (size_t)n_mat);   /* one call: consecutive ops share sweeps */
+    if (!rc && n_ch) rc = qsb_apply_channels(s, chs, (size_t)n_ch, ch_r, ch_b, ch_p);   /* one call: channels share sweeps */
     if (!rc && (n_rot || n_gterm)) {   /* one call for all rotations: consecutive ones share sweeps over the state */
         uint64_t *rx = (uint64_t *)malloc(sizeof(uint64_t) * 2 * (n_rot + n_gterm) + 16);
         if (!rx) { printf("Malloc error\n"); return 1; }
@@ -237,6 +289,11 @@ int main(int argc, char **argv)
                nq, (unsigned long long)st.source_gates, st.passes, st.rounds, st.device_ms, st.plan_ms,
                (unsigned long long)st.bytes_moved, st.device_ms > 0 ? st.bytes_moved / st.device_ms * 1e-6 : 0.0,
                st.device_ms > 0 ? st.source_gates / st.device_ms * 1e3 : 0.0);
+    }
+    for (int m = 0; m < n_ch; m++) {
+        printf("CHANNEL");
+        for (int i = 0; i < chs[m].k; i++) printf(" %d", chs[m].targets[i]);
+        printf(": %u %.17g\n", ch_b[m], ch_p[m]);
     }
     if (n_gterm) {
         printf("ENERGY %.17g\n", energy);
@@ -347,6 +404,13 @@ int main(int argc, char **argv)
     free(grad);
     for (int m = 0; m < n_mat; m++) free((void *)mops[m].m);
     free(mops);
+    for (int m = 0; m < n_ch; m++) free((void *)chs[m].kraus);
+    free(chs);
+    free(ch_r);
+    free(ch_p);
+    free(ch_b);
+    free(ch_q);
+    free(ch_f);
     free(mat_q);
     free(mat_f);
     return 0;

@@ -403,7 +403,9 @@ int collapse_pass(qsb_sim *s, const Geom &G, uint64_t outcome, double p)
     return QSB_OK;
 }
 
-/* the rule of measurement() (quantum_simulator.c:279) on the table: first b with C_b != 0 and C_b >= r * T */
+}  // namespace
+
+/* declared in sim.h */
 int pick_outcome(const std::vector<double> &tab, double r, uint64_t *b_out, const char *fn)
 {
     double T = 0.0;
@@ -418,6 +420,8 @@ int pick_outcome(const std::vector<double> &tab, double r, uint64_t *b_out, cons
     *b_out = tab.size() - 1;   /* not reached: C_last = T >= r * T and T != 0 */
     return QSB_OK;
 }
+
+namespace {
 
 int measure_common(qsb_sim *s, const int *qubits, int k, double r, uint64_t *outcome, double *prob, const char *fn)
 {

@@ -57,5 +57,9 @@ int qsb_canonicalise(const qsb_gate_t *gates, size_t n, int num_qubits, std::vec
  * min(n, kmax); hint says what to do about a k above kmax */
 int check_qubits(const qsb_sim *s, const int *qubits, int k, int kmax, const char *fn, const char *hint);
 
+/* the rule of measurement() (quantum_simulator.c:279) on a table of weights: the first b whose inclusive serial fp64
+ * prefix sum C_b is != 0 and >= r * T, T = the sum of the table; QSB_ERR_ARG (with a message naming fn) if T is not > 0 */
+int pick_outcome(const std::vector<double> &tab, double r, uint64_t *b_out, const char *fn);
+
 /* element size of one amplitude */
 static inline size_t amp_bytes(int prec) { return prec == QSB_F64 ? 16 : 8; }

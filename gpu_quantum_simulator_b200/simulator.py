@@ -13,7 +13,7 @@ import os
 
 import numpy as np
 
-from ._lib import lib, check, Gate, MatrixOp, Options, RunStats, F32, F64, MODE_TILED, MODE_SWEEP
+from ._lib import lib, check, Gate, MatrixOp, Channel, Options, RunStats, F32, F64, MODE_TILED, MODE_SWEEP
 
 
 def _gate_array(gates):
@@ -204,6 +204,83 @@ def overlap_dry_run(num_qubits, perm_a, perm_b, precision_a=F32, precision_b=F32
     check(lib.qsb_inner_product_dry_run(num_qubits, C.byref(oa), pa.ctypes.data, C.byref(ob), pb.ctypes.data, C.byref(st),
                                         C.byref(ex)))
     return {"steps": st.value, "exchanges": ex.value}
+
+
+def _channels(channels):
+    """[(kraus_list, qubits)] -> (ctypes array of Channel, the numpy buffers its pointers address).  kraus_list is None in
+    a dry run (the channel is then taken as state-dependent); otherwise a list of (2^k, 2^k) complex arrays."""
+    arr = (Channel * max(len(channels), 1))()
+    keep = []
+    for i, (kraus, qubits) in enumerate(channels):
+        qubits = [int(x) for x in np.atleast_1d(qubits)]
+        if len(qubits) > 4:
+            raise ValueError(f"channel {i}: {len(qubits)} targets, at most 4")
+        c = arr[i]
+        c.k = len(qubits)
+        for j, x in enumerate(qubits):
+            c.targets[j] = x
+        if kraus is None:
+            c.nkraus = 1                        # shapes only: the count is checked, the operators are not read
+            continue
+        d = 1 << len(qubits)
+        ks = np.ascontiguousarray(np.asarray(kraus, dtype=np.complex128))
+        if ks.ndim != 3 or ks.shape[1:] != (d, d):
+            raise ValueError(f"channel {i}: Kraus operators of shape {ks.shape} for {len(qubits)} targets, expected (m, {d}, {d})")
+        c.nkraus = ks.shape[0]
+        keep.append(ks)
+        c.kraus = ks.view(np.float64).ctypes.data_as(C.POINTER(C.c_double))
+    return arr, keep
+
+
+def channel_dry_run(num_qubits, channels, precision=F32, world_size=1, low_bits=0):
+    """Host-only: {"sweeps", "gram_sweeps", "exchanges"} that Simulator.apply_channels would run for these channels from the
+    identity qubit layout, counting every branch as a non-identity operator (an upper bound): sweeps = launches that read
+    and write the local shard, gram_sweeps = launches that only read it, exchanges = partner shards fetched.  channels:
+    (kraus_list, qubits) tuples as for apply_channels; kraus_list may be None (taken as state-dependent), and a qubit list
+    that is not a tuple stands for (None, qubits)."""
+    chs = [c if isinstance(c, tuple) else (None, c) for c in channels]
+    arr, keep = _channels(chs)
+    o = _options(precision, MODE_TILED, low_bits, 0, world_size, -1)
+    sw, gs, ex = C.c_uint32(), C.c_uint32(), C.c_uint32()
+    check(lib.qsb_channel_dry_run(num_qubits, C.byref(o), arr, len(chs), C.byref(sw), C.byref(gs), C.byref(ex)))
+    del keep
+    return {"sweeps": sw.value, "gram_sweeps": gs.value, "exchanges": ex.value}
+
+
+_PAULI = [np.eye(2, dtype=np.complex128), np.array([[0, 1], [1, 0]], dtype=np.complex128),
+          np.array([[0, -1j], [1j, 0]], dtype=np.complex128), np.array([[1, 0], [0, -1]], dtype=np.complex128)]
+
+
+def depolarizing(p, k=1):
+    """Kraus operators of the k-qubit depolarizing channel rho -> (1 - p) rho + p I / 2^k (k = 1 or 2): sqrt(1 - p (4^k - 1)
+    / 4^k) I and sqrt(p / 4^k) P for every other Pauli product P (bit i of an index = qubit i of the channel's list)."""
+    if k not in (1, 2):
+        raise ValueError(f"depolarizing: k = {k}, expected 1 or 2")
+    d2 = 4 ** k
+    ops = []
+    for idx in range(d2):
+        P = np.ones((1, 1), dtype=np.complex128)
+        for j in range(k):                      # qubit j is bit j of the index: kron(P_{k-1}, ..., P_0)
+            P = np.kron(_PAULI[(idx >> (2 * j)) & 3], P)
+        ops.append(P * np.sqrt(1.0 - p * (d2 - 1) / d2 if idx == 0 else p / d2))
+    return ops
+
+
+def pauli_channel(px, py, pz):
+    """Kraus operators of rho -> (1 - px - py - pz) rho + px X rho X + py Y rho Y + pz Z rho Z."""
+    return [np.sqrt(1.0 - px - py - pz) * _PAULI[0], np.sqrt(px) * _PAULI[1], np.sqrt(py) * _PAULI[2], np.sqrt(pz) * _PAULI[3]]
+
+
+def amplitude_damping(gamma):
+    """Kraus operators of amplitude damping: [[1, 0], [0, sqrt(1 - gamma)]] and [[0, sqrt(gamma)], [0, 0]]."""
+    return [np.array([[1, 0], [0, np.sqrt(1.0 - gamma)]], dtype=np.complex128),
+            np.array([[0, np.sqrt(gamma)], [0, 0]], dtype=np.complex128)]
+
+
+def phase_damping(lam):
+    """Kraus operators of phase damping: [[1, 0], [0, sqrt(1 - lam)]] and [[0, 0], [0, sqrt(lam)]]."""
+    return [np.array([[1, 0], [0, np.sqrt(1.0 - lam)]], dtype=np.complex128),
+            np.array([[0, 0], [0, np.sqrt(lam)]], dtype=np.complex128)]
 
 
 class Plan:
@@ -439,6 +516,30 @@ class Simulator:
         arr, keep = _matrix_ops(ops)
         check(lib.qsb_apply_matrices(self._h, arr, len(ops)))
         del keep
+
+    # ---- noise channels (bit i of a row or column index of a Kraus operator is the value of qubits[i])
+    def apply_channels(self, channels, r=None, seed=0):
+        """Quantum trajectories: for each (kraus_list, qubits) in list order, pick branch i with probability
+        w_i / T = ||K_i psi||^2 / sum_j ||K_j psi||^2 (the first i whose prefix sum reaches r[c] * T) and apply
+        sqrt(T / w_i) K_i, on the device.  r defaults to sample_uniform(seed, c) for channel c.  Returns (branch uint32
+        array, prob float64 array).  Sharded: collective, same arguments (r included) on every rank."""
+        chs = list(channels)
+        if r is None:
+            r = [sample_uniform(seed, c) for c in range(len(chs))]
+        rr = np.ascontiguousarray(np.asarray(r, dtype=np.float64).reshape(-1))
+        if rr.size != len(chs):
+            raise ValueError(f"{len(chs)} channels but {rr.size} values of r")
+        arr, keep = _channels(chs)
+        branch = np.zeros(len(chs), dtype=np.uint32)
+        prob = np.zeros(len(chs), dtype=np.float64)
+        check(lib.qsb_apply_channels(self._h, arr, len(chs), rr.ctypes.data, branch.ctypes.data, prob.ctypes.data))
+        del keep
+        return branch, prob
+
+    def apply_channel(self, kraus, qubits, r):
+        """One channel: returns (branch, prob) as an int and a float."""
+        b, p = self.apply_channels([(kraus, qubits)], [r])
+        return int(b[0]), float(p[0])
 
     # ---- marginals and projective measurement (bit i of a bin index or an outcome is the value of qubits[i])
     @staticmethod

@@ -398,6 +398,59 @@ int qsb_copy_state(qsb_t *dst, const qsb_t *src);
 int qsb_inner_product_dry_run(int num_qubits, const qsb_options_t *opt_a, const int8_t *perm_a,
                               const qsb_options_t *opt_b, const int8_t *perm_b, uint32_t *steps, uint32_t *exchanges);
 
+/* ---- noise channels -----------------------------------------------------------
+ * Quantum trajectories: a channel is a set of Kraus operators {K_i} on k distinct LOGICAL target qubits, 1 <= k <=
+ * QSB_CHANNEL_MAX_K, each K_i a 2^k x 2^k complex matrix in the m format of qsb_matrix_op_t (bit i of a row / column
+ * index = value of targets[i]).  qsb_apply_channels applies ch[0..n-1] in list order (the first listed acts first; no
+ * channel is reordered).  For channel c, on the state as it stands after channels 0..c-1:
+ *   - w_i = ||K_i psi||^2 in fp64, summed in a fixed order, T = sum_i w_i (the norm for a trace-preserving set);
+ *   - branch[c] = the first i whose inclusive prefix sum C_i is != 0 and >= r[c] * T (the rule of qsb_measure_qubits);
+ *   - prob[c] = w_i / T (prob may be NULL);
+ *   - psi <- sqrt(T / w_i) K_i psi: the norm is kept, not forced to 1, so a branch of a mixed-unitary channel is applied
+ *     as exactly its unitary.
+ * Fixed-weight channels: when every K_i^dag K_i is within 1e-12 (max abs entry) of q_i I, q_i = Tr(K_i^dag K_i) / 2^k
+ * (Pauli channels, depolarizing, bit and phase flip), w_i / T is taken as q_i on the host without reading the state:
+ * prob[c] = q_i and the applied matrix is K_i / sqrt(q_i).  A chosen operator that is a positive real multiple of the
+ * identity (imaginary parts and off-diagonal entries exactly 0, equal positive diagonal) changes no byte of the state.
+ *
+ * Applied on the device in groups (DESIGN.md section 3.3, noise channels).  The chosen operators wait in a pending run.
+ * A state-dependent channel starts a group that takes the following channels while the union U of their targets has at
+ * most 4 qubits.  The pending run is applied as one qsb_apply_matrices call, and the group reads rho_U, the reduced
+ * density matrix of U, with one qsb_reduced_density_matrix call.  The channels of the group are then resolved on the
+ * host in fp64, in order: w_i = Re Tr(K_i rho K_i^dag), the branch, rho <- (T / w_i) K_i rho K_i^dag.  So the weights of
+ * the second and later channels of a group come from rho_U carried on the host, not from a new read of the state; for
+ * f32 states this differs from a fresh read by the rounding of the applied ops only.  Both calls are deterministic:
+ * repeated calls return identical bits.
+ * Errors return QSB_ERR_ARG with the state untouched, checked on the host before anything is launched: a null handle,
+ * a null ch, r or branch when n > 0, k outside [1, min(n_qubits, QSB_CHANNEL_MAX_K)], a target >= n_qubits or repeated,
+ * nkraus outside [1, 4^k], a null kraus, a non-finite entry, flags != 0, an r outside [0, 1) or NaN, a set that is not
+ * trace-preserving (max abs entry of sum_i K_i^dag K_i - I above 1e-10), a low_bits outside the range the tile scheduler
+ * accepts (as for qsb_apply_matrices).  A state of norm 0 at a weight read gives QSB_ERR_ARG and is still the zero
+ * vector.  n = 0 is a no-op.  A sharded handle without qsb_comm_init gives QSB_ERR_COMM.
+ * The qubit layout, the state buffer (a captured graph's state), the role of the exchange buffer and the peer mappings
+ * are left as they are, so a plan made before the call still executes after it.
+ * On a sharded state the call is collective (the same arguments, r included, on every rank) and every rank gets the same
+ * branches and probabilities, bit for bit, since rho_U is the same on every rank; rank targets cost the partner-shard
+ * copies of those two calls. */
+#define QSB_CHANNEL_MAX_K 4
+typedef struct qsb_channel {
+    int32_t k;                           /* targets, 1..QSB_CHANNEL_MAX_K */
+    int32_t targets[QSB_CHANNEL_MAX_K];  /* distinct logical qubits; bit i of a row / column index = value of targets[i] */
+    int32_t nkraus;                      /* Kraus operators, 1..4^k */
+    int32_t flags;                       /* reserved, 0 */
+    const double *kraus;                 /* nkraus operators of 2 * 4^k doubles each, each in the m format of
+                                            qsb_matrix_op_t (row-major re, im); operator i at kraus + i * 2 * 4^k */
+} qsb_channel_t;
+
+int qsb_apply_channels(qsb_t *s, const qsb_channel_t *ch, size_t n, const double *r, uint32_t *branch, double *prob);
+/* Host only, no device, from the identity layout: the sweeps that write the shard (those of qsb_matrix_dry_run for each
+ * pending run), the reads of rho_U (gram_sweeps: 2^m for a group with m qubits on rank bits) and the partner-shard copies
+ * of both (exchanges) that qsb_apply_channels would run.  kraus may be NULL: that
+ * channel is then taken as state-dependent.  Every branch is counted as a non-identity operator, so the numbers are an
+ * upper bound.  The argument checks are those of qsb_apply_channels (r is not read). */
+int qsb_channel_dry_run(int num_qubits, const qsb_options_t *opt, const qsb_channel_t *ch, size_t n,
+                        uint32_t *sweeps, uint32_t *gram_sweeps, uint32_t *exchanges);
+
 /* ---- shard dump / reload ----------------------------------------------------
  * The reference keeps the state only in memory (quantum_simulator.c:75 frees it
  * at exit); long sharded runs want a checkpoint.  File = 128-byte header (magic
